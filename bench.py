@@ -6,8 +6,9 @@ Workload = config c3 of BASELINE.json exactly ("Batched likelihood sweep: 65,536
 sharded over 1/2/4/8 B200"): SubjectiveActor 2-D tracking, N=100 trials x T=1200, a sweep of 65,536 parameter samples IN
 TOTAL, sharded over the GPUs by parameter samples (STRONG scaling: every rank evaluates 65,536 / n_gpus samples).  One
 "step" = one log-likelihood + parameter-gradient evaluation of all 65,536 samples (6,553,600 trial evals).  Data are
-synthetic: the GPU legs simulate them with the product's own System.simulate (torch Philox, seed 7), the CPU legs with the
-oracle's restatement (NumPy PCG64, seed 7); parameter samples are theta_true * exp(0.25 z), z ~ N(0, I_6), seed 11.
+synthetic: the c3 legs (GPU and CPU) take them from the oracle's restatement of System.simulate (NumPy PCG64, seed 7), the
+secondary GPU workloads from the product's own System.simulate (torch Philox); parameter samples are
+theta_true * exp(0.25 z), z ~ N(0, I_6), seed 11.
 
   value : device-resident (base matrices + observations already in HBM) through the C ABI, CUDA events, max over ranks;
           every rank ends the step with the complete sweep result (all-gather of the per-sample [ll, base-matrix gradients]
@@ -25,6 +26,8 @@ oracle's restatement (NumPy PCG64, seed 7); parameter samples are theta_true * e
           [ll, grad]), c5 (one leapfrog of 4,096 lock-step chains, chains sharded over the ranks) at every N; c4 at N=1.
 
 `--impl reference` runs only the CPU port (the real JAX reference is not installable in this image).
+`--dump-outputs DIR` writes what the last timed step of the value and e2e legs computed as DIR/<name>.npy; the inputs of
+those legs come from seeded NumPy generators only, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -93,7 +96,7 @@ def source_sha():
 
 # ----------------------------------------------------------------------------------------------- helpers
 def make_data(N, T, seed=7):
-    """Synthetic tracking data for the CPU legs: float64 restatement of System.simulate (oracle), NumPy PCG64."""
+    """Synthetic tracking data for the c3 legs: float64 restatement of System.simulate (oracle), NumPy PCG64."""
     from oracle import lqg_np as O
     kw = dict(zip(PARAM_NAMES, THETA_TRUE))
     sa, sd = O.make_system(O.subjective_actor_mats(dim=2, **kw), T)
@@ -101,8 +104,8 @@ def make_data(N, T, seed=7):
 
 
 def make_data_gpu(N, T, dev, seed=7, **overrides):
-    """Synthetic tracking data for the GPU legs from the product's own simulator (lqg_b200 System.simulate, torch Philox);
-    the oracle is not involved in anything the GPU legs measure."""
+    """Synthetic tracking data for the secondary GPU workloads from the product's own simulator (lqg_b200 System.simulate,
+    torch Philox)."""
     from lqg_b200.tracking import SubjectiveActor
     kw = dict(zip(PARAM_NAMES, THETA_TRUE))
     kw.update(overrides)
@@ -180,6 +183,24 @@ def cpu_port_eval(S, N, T, X, seed=3):
     ll.sum().backward()
     assert torch.isfinite(th.grad).all()
     return time.perf_counter() - t0
+
+
+DUMP_MAX_BYTES = 16 << 20      # per array of --dump-outputs (three arrays: at most 48 MiB in all)
+
+
+def dump(out_dir, **arrays):
+    """--dump-outputs: every tensor as out_dir/<name>.npy in its own dtype (float32 / float64).  An array larger than
+    DUMP_MAX_BYTES keeps a fixed, seeded sample of its rows (NumPy default_rng(0), in row order), so that runs with the same
+    arguments write the same elements and two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        keep = max(1, DUMP_MAX_BYTES // (t[0].numel() * t.element_size()))
+        if t.shape[0] > keep:
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        a = t.detach().cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def timed(fn, reps, warm, barrier):
@@ -440,8 +461,8 @@ def run_ours(args):
     # ---------------- device-resident leg (C ABI)
     theta = torch.tensor(theta_np, device=dev)
     model = SubjectiveActor(dim=2, T=T, device=dev, **{n: theta[:, i] for i, n in enumerate(PARAM_NAMES)})
-    x_dev = make_data_gpu(N, T, dev)
-    X = x_dev.cpu().numpy()
+    X = make_data(N, T)                               # seeded NumPy, so the inputs do not depend on the build being timed
+    x_dev = torch.tensor(X, device=dev)
     if args.no_factorize:
         sysm, xk, Nk = model, x_dev, N
         dims = abi.LqgkDims(S, N, T, DIMS["x"], DIMS["b"], DIMS["u"], DIMS["y"], DIMS["d"])
@@ -464,7 +485,7 @@ def run_ours(args):
         # the sweep result of this rank: per sample [sum_i ll_i, all base-matrix gradients]; gathered so that every rank holds
         # the complete sweep (the path's one collective, lqg_b200.parallel)
         packed = torch.cat([ll.sum(1, keepdim=True)] + [g.reshape(S, -1) for g in list(ga.values()) + list(gd.values())], 1)
-        return parallel.gather_samples(packed, S_total)
+        return parallel.gather_samples(packed, S_total), ll
 
     def barrier():
         torch.cuda.synchronize()
@@ -475,7 +496,7 @@ def run_ours(args):
     sampler = ClockSampler(local)
     sampler.start()                                   # started before the warm-up so samples exist when the timed region begins
     for _ in range(args.warmup):
-        res = step_resident()
+        res, ll_trials = step_resident()
     barrier()
     launches_per_step = lib.last_launch_count()
     lib.profile_enable(True)
@@ -484,7 +505,7 @@ def run_ours(args):
     sampler.mark_start()
     e0.record()
     for _ in range(args.steps):
-        res = step_resident()
+        res, ll_trials = step_resident()
     e1.record()
     barrier()
     sampler.mark_end()
@@ -492,6 +513,16 @@ def run_ours(args):
     prof = lib.profile_read()
     lib.profile_enable(False)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # sweep[S_total, 1 + G]: per parameter sample [sum_i ll_i, the actor's (A B F V W Q R) and the dynamics' (A B F V W)
+        # base-matrix gradients, each row-major] -- what every rank holds after the step.  ll[S_total, N]: per-trial
+        # log-likelihoods in the public API's layout (the axes the factorised kernels see as separate trials summed back into
+        # one trial, as SubjectiveActor.log_likelihood does), gathered from all ranks.
+        ll = parallel.gather_samples(ll_trials.reshape(S, -1, N).sum(1), S_total)
+        if rank == 0:
+            dump(args.dump_outputs, sweep=res, ll=ll)
+        del ll
+    del ll_trials
     # The pipelined launch sequence overlaps kernels of different streams, so the per-kernel event times above include the
     # time a kernel shares the SMs with others.  Two extra steps (outside the timed region) with the plain sequence give
     # every kernel's time when it runs alone -- reported next to the live numbers.
@@ -533,9 +564,11 @@ def run_ours(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step_e2e()
+        full = step_e2e()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump(args.dump_outputs, e2e_ll_grad=full)                  # [S_total, 1 + 6]: sum_i ll_i, d/dtheta (PARAM_NAMES order)
     t_e = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t_e, op=dist.ReduceOp.MAX)
@@ -772,7 +805,11 @@ def main():
     ap.add_argument("--pipe-max", type=int, default=-1, help="largest chunk (samples) that uses the pipelined launch sequence; -1 = library default")
     ap.add_argument("--pipe-segments", type=int, default=6)
     ap.add_argument("--no-factorize", action="store_true", help="run the general 2-D (n=10) kernels instead of the per-axis factorisation")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (device-resident sweep and "
+                                                          "per-trial log-likelihoods, end-to-end ll + gradient) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -93,7 +93,7 @@ def test_predictive_moments(host, name, cls, kw):
     T, N = 40, 3
     mats = H.model_mats(name)
     X = _sim(mats, T, N, seed=3).astype(np.float32)
-    model = cls(T=T, dtype=torch.float64, **kw)
+    model = cls(T=T, dtype=torch.float64, device="cpu", **kw)
     mu, Sig = runtime.moments(model.actor, model.dynamics, torch.tensor(X))
     sa, sd = O.make_system(mats, T)
     for i in range(N):

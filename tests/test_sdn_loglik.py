@@ -159,7 +159,7 @@ def test_channel_noise_matches_its_numpy_twin():
     from lqg_b200.control import sdn
     from lqg_b200.tracking import SubjectiveActor
     for dim in (1, 2):
-        model = SubjectiveActor(dim=dim, T=10, dtype=torch.float64)
+        model = SubjectiveActor(dim=dim, T=10, dtype=torch.float64, device="cpu")
         _, sa, sd, _, _ = _system("subjective" if dim == 1 else "subjective2", T=10)
         C, D = _channel_noise_np(sd, 3.0, 0.25)
         assert np.allclose(sdn.channel_noise(model, 3.0, "control").numpy(), np.stack(C))
@@ -295,7 +295,7 @@ def test_python_api_with_sdn_aware_actor_on_host(monkeypatch):
     from lqg_b200.tracking import SubjectiveActor
     _route_python_api_to_host_harness(monkeypatch)
     T_ = 40
-    model = SubjectiveActor(dim=2, T=T_, dtype=torch.float64)
+    model = SubjectiveActor(dim=2, T=T_, dtype=torch.float64, device="cpu")
     _, sa, sd, _, _ = _system("subjective2", T=T_)
     Ca, Da = _channel_noise_np(sa, 40.0, 0.4)                       # the actor's own input / observation maps
     A0 = {k: sa[k][0] for k in "ABFVWQR"}
