@@ -209,15 +209,16 @@ int lqgk_init(int max_sample_slices);
 /* Number of internal concurrent sample slices (streams) used by the likelihood entry points of the calling thread
  * (default 1 = everything on the caller's stream; 4 gives ~3 % at the benchmark size, see DESIGN.md).  Work is always forked from / joined to the caller's stream. */
 int lqgk_set_streams(int n);
-/* Run the independent kernels of one chunk (lqr_fwd | kf_fwd, the two contraction passes, kf_rev | lqr_rev | reduction)
- * concurrently on internal auxiliary streams.  mask bit 0: lqr_fwd | kf_fwd, bit 1: contraction passes, bit 2: adjoint tail;
- * default 6. */
+/* Kernel overlap inside one call: 0 keeps every chunk on one stream (no internal auxiliary streams); any other value
+ * (1..7, default 6) lets the fused forward+adjoint call run the pipelined launch sequence of lqgk_set_pipeline over internal
+ * auxiliary streams. */
 int lqgk_set_kernel_overlap(int mask);
 /* Pipelined launch sequence of the fused forward+adjoint call: chunks of at most `max_samples` parameter samples (default:
  * no limit; 0 = never) cut every sweep over time into `segments` segments (default 6) and run the sweeps of one direction as a
  * software pipeline over the internal streams (kf_fwd -> cov_fwd -> trial_fwd, then trial_rev -> cov_seq_rev -> contraction ->
  * kf_rev): at small sample counts every sweep is latency-bound and the chain of nine sweeps, not the arithmetic, sets the time of
- * one evaluation (a NUTS leapfrog).  Results do not depend on the setting beyond FP64 summation order. */
+ * one evaluation (a NUTS leapfrog).  Otherwise the same sequence runs as one segment on the chunk's stream, as do forward-only
+ * calls and systems with joint dim > 12.  Results do not depend on the setting beyond FP64 summation order. */
 int lqgk_set_pipeline(int max_samples, int segments);
 /* Tuning knob: target number of (32-sample group x time-range) warps of the time-parallel contraction kernels. */
 int lqgk_set_contrib_warps(int n);

@@ -420,7 +420,7 @@ const char* lqgk_strerror(int code) {
 }
 int lqgk_init(int max_sample_slices) {
   // everything an entry point may need later on this thread and device, created now: the internal streams / events (sample
-  // slices + 2 auxiliary streams per slice) and the cached SM count.  After this no entry point creates CUDA objects, so calls
+  // slices + 3 auxiliary streams per slice) and the cached SM count.  After this no entry point creates CUDA objects, so calls
   // may be captured into CUDA graphs (which is how XLA may run an FFI handler).
   if (max_sample_slices < 1 || max_sample_slices > 32) return LQGK_E_INVALID;
   sm_count();

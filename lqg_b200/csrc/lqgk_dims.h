@@ -12,7 +12,7 @@
   M(4, 4, 1, 3, 2)   /* PointMassBoundedActor, observed target+cursor (point_mass.py, main.py:51) */ \
   M(5, 5, 1, 2, 2)   /* HandMotionModelTrackingTask (notebooks/HandModel.ipynb): target + pos/vel/force/act. */ \
   M(6, 6, 1, 2, 2)   /* TemporalDelayModel(BoundedActor dim=1, delay=2) (delay.py:9-41): motor-delay family */ \
-  M(12, 12, 1, 3, 2) /* TemporalDelayModel(PointMassBoundedActor, delay=2): 12-dim state, joint dim 24 [config c4]; large-system path (lqgk_big.cuh) */
+  M(12, 12, 1, 3, 2) /* TemporalDelayModel(PointMassBoundedActor, delay=2): 12-dim state, joint dim 24 [config c4]; large-system kernels (lqgk_bigw.cuh) */
 // Tuples compiled ONLY for the all-FP64 per-trial likelihood (k_sdn_loglik: lqgk_sdn_loglik_*, System.log_likelihood_fp64): models
 // whose innovation covariance is too ill-conditioned for the FP32 per-trial arithmetic of the main path (DESIGN.md section 7).
 #define LQGK_FOR_EACH_FP64_ONLY_DIMS(M)                                                                      \

@@ -1,6 +1,6 @@
 // lqgk_inst.cu -- instantiates every kernel and the launch sequence for ONE dimension tuple, selected with
 // -DLQGK_INST_X/B/U/Y/D (one object file per line of lqgk_dims.h; __graft_entry__.build() compiles them in parallel).
-#include "lqgk_big.cuh"
+#include "lqgk_run.cuh"
 
 #if !defined(LQGK_INST_X)
 #error "compile with -DLQGK_INST_X=.. -DLQGK_INST_B=.. -DLQGK_INST_U=.. -DLQGK_INST_Y=.. -DLQGK_INST_D=.."
@@ -10,15 +10,13 @@ namespace lqgk {
 using DMI = Dims<LQGK_INST_X, LQGK_INST_B, LQGK_INST_U, LQGK_INST_Y, LQGK_INST_D>;
 #if defined(LQGK_BIG)
 static_assert(is_big<DMI>(), "-DLQGK_BIG is for joint dims > 12 only");
-template <class T> static int run_sel(const Call& c) { return run_big<DMI, T>(c); }
 #else
 static_assert(!is_big<DMI>(), "joint dims > 12 must be compiled with -DLQGK_BIG");
-template <class T> static int run_sel(const Call& c) { return run<DMI, T>(c); }
 #endif
 template <>
-int Runner<LQGK_INST_X, LQGK_INST_B, LQGK_INST_U, LQGK_INST_Y, LQGK_INST_D>::run_f32(const Call& c) { return run_sel<float>(c); }
+int Runner<LQGK_INST_X, LQGK_INST_B, LQGK_INST_U, LQGK_INST_Y, LQGK_INST_D>::run_f32(const Call& c) { return run<DMI, float>(c); }
 template <>
-int Runner<LQGK_INST_X, LQGK_INST_B, LQGK_INST_U, LQGK_INST_Y, LQGK_INST_D>::run_f64(const Call& c) { return run_sel<double>(c); }
+int Runner<LQGK_INST_X, LQGK_INST_B, LQGK_INST_U, LQGK_INST_Y, LQGK_INST_D>::run_f64(const Call& c) { return run<DMI, double>(c); }
 template <>
 size_t Runner<LQGK_INST_X, LQGK_INST_B, LQGK_INST_U, LQGK_INST_Y, LQGK_INST_D>::plan_bytes(const LqgkDims& d, int mode, int32_t max_chunk) {
   size_t Sc = choose_chunk<DMI>(d, mode, false, (size_t)-1, max_chunk);

@@ -31,7 +31,7 @@ extern thread_local Profiler g_prof;
 // streams (forked from / joined to the caller's stream with events); each slice owns a part of the workspace.
 extern thread_local int g_streams;
 extern thread_local int g_contrib_warps;   // target number of (sample-group x time-range) warps of the contraction kernels
-extern thread_local int g_aux_streams;   // bit 0: lqr_fwd | kf_fwd, bit 1: contraction passes, bit 2: kf_rev | lqr_rev | reduce
+extern thread_local int g_aux_streams;   // 0: no internal auxiliary streams (no pipelined launch sequence); else allowed
 // SM count of the calling thread's current device (queried once per device, never hard-coded): sizes the grids of the
 // time-parallel kernels.
 struct DeviceInfo {
@@ -151,7 +151,7 @@ inline bool spec_time_varying(const LqgkSpec& s, bool actor) {
   return false;
 }
 
-// Large systems (joint dim > 12) take the local-memory path of lqgk_big.cuh (compiled with -DLQGK_BIG).
+// Large systems (joint dim > 12) take the warp-per-sample kernels of lqgk_bigw.cuh (see the kernel launchers below).
 template <class DM>
 constexpr bool is_big() { return DM::N > 12; }
 // Workspace plan for one chunk of Sc (multiple of 32) samples.
@@ -238,29 +238,13 @@ int set_smem(const void* fn, size_t bytes) {
   return LQGK_OK;
 }
 
-// Observations of one chunk in the per-trial kernels' component-major layout (k_repack_obs): one data set shared by all
-// samples (x_sample_stride == 0) or one per sample of the chunk.  Returns the element stride between the data sets in xc.
-inline int launch_repack_obs(cudaStream_t st, const LqgkDims& d, int row, const float* x_tm, int s0, int n, float* xc, size_t* xc_stride) {
-  const int nb = (d.N + row - 1) / row;
-  const bool per_sample = d.x_sample_stride != 0;
-  const size_t per = (size_t)(d.T + 1) * nb * d.d * row;
-  const int nsets = per_sample ? n : 1;
-  *xc_stride = per_sample ? per : 0;
-  const size_t total = per * nsets;
-  const unsigned blocks = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)sm_count() * 16);
-  ProfScope ps_(PK_PACK, st);
-  k_repack_obs<float><<<blocks, 256, 0, st>>>(x_tm, (size_t)d.x_sample_stride, per_sample ? s0 : 0, nsets, d.N, row, d.T + 1, d.d, xc);
-  LQGK_LAUNCH_CHECK();
-  return LQGK_OK;
-}
-// ka, kb: range of checkpoint segments of this launch (kb < 0: all of them)
+// ka, kb: range of checkpoint segments of this launch
 template <class DM, int RT>
 int launch_trial_fwd(cudaStream_t st, const float* rec, const float* xc, size_t xcs, int n, int N, int T, double* ll, float* hist,
-                     int ka = 0, int kb = -1) {
+                     int ka, int kb) {
   size_t smem = trial_smem_bytes<DM, RT, false>();
   int rc = set_smem<DM>((const void*)k_trial_fwd<DM, RT>, smem);
   if (rc) return rc;
-  if (kb < 0) kb = (T + trial_ck<DM>(RT) - 1) / trial_ck<DM>(RT);
   ProfScope ps_(PK_TRIAL_FWD, st);
   k_trial_fwd<DM, RT><<<(n + TRIAL_WARPS - 1) / TRIAL_WARPS, 32 * TRIAL_WARPS, smem, st>>>(rec, xc, xcs, n, N, T, ll, hist, ka, kb);
   LQGK_LAUNCH_CHECK();
@@ -268,11 +252,10 @@ int launch_trial_fwd(cudaStream_t st, const float* rec, const float* xc, size_t 
 }
 template <class DM, int RT>
 int launch_trial_rev(cudaStream_t st, const float* rec, const float* xc, size_t xcs, const float* hist, const float* w, int n, int N, int T,
-                     float* sums, float* cbcar, int ka = 0, int kb = -1) {
+                     float* sums, float* cbcar, int ka, int kb) {
   size_t smem = trial_smem_bytes<DM, RT, true>();
   int rc = set_smem<DM>((const void*)k_trial_rev<DM, RT>, smem);
   if (rc) return rc;
-  if (kb < 0) kb = (T + trial_ck<DM>(RT) - 1) / trial_ck<DM>(RT);
   ProfScope ps_(PK_TRIAL_REV, st);
   k_trial_rev<DM, RT><<<(n + TRIAL_WARPS_REV - 1) / TRIAL_WARPS_REV, 32 * TRIAL_WARPS_REV, smem, st>>>(rec, xc, xcs, hist, w, n, N, T, sums, ka,
                                                                                                      kb, cbcar);
@@ -300,13 +283,326 @@ struct Call {
   void *mu_out = nullptr, *Sig_out = nullptr;   // moments entry point
 };
 
+// ------------------------------------------------------------------------------------------------------- kernel launchers
+// One launcher per stage of the likelihood path.  A launcher takes its stream and, for a sweep over time, the range of one
+// pipeline segment ([t0, t1) in steps; [ka, kb) in checkpoint segments for the per-trial kernels).  It picks the kernel variant
+// for the system size and the covariance mapping, sets the kernel's dynamic shared memory, times the launch (ProfScope) and
+// checks it.
+//
+// Small systems (joint dim n <= 12) keep every matrix of a sample in registers (one thread per sample, fully unrolled
+// templates) and its constants in shared memory, with sample-minor workspace arrays.  Few samples (a handful of conditions, a
+// few hundred chains per GPU) leave the thread-per-sample covariance kernels with an idle GPU and every step costing one thread's
+// instruction stream; calls with at most g_warp_cov_max_samples samples therefore run the large systems' warp-per-sample
+// covariance kernels, which spread a step over 32 lanes (S = 8: covariance forward 3.3 -> 2.4 ms, sequential adjoint
+// 2.5 -> 1.0 ms) and win up to ~1,000 samples.  The Riccati / Kalman sweeps stay thread-per-sample (3 x 3 products do not
+// spread), hence GAINS_MINOR: the warp kernels read the sample-minor gains of those sweeps.
+//
+// Large systems (joint dim n > 12, e.g. the 24-dim delayed point-mass model of BASELINE config c4:
+// TemporalDelayModel(PointMassBoundedActor, delay=2)): neither fits at n = 24 (576-entry joint matrices, ~900 derived
+// constants per sample), and these systems come in thousands, not hundreds of thousands, of samples.  Their path therefore
+// maps ONE WARP PER PARAMETER SAMPLE with the matrices in shared memory (lqgk_bigw.cuh: kw_lqr_fwd, kw_kf_fwd, kw_cov_fwd,
+// kw_cov_seq_rev, kw_cov_contrib, kw_kf_rev, kw_lqr_rev) and sample-major workspace arrays.  The per-trial FP32 kernels
+// (k_trial_fwd / k_trial_rev: warp per sample, lane = trial, TMA-staged records) are shared with the small-system path; only
+// their ring geometry adapts to the record size.  The object is compiled with -DLQGK_BIG (rolled FP64 loops in the scalar
+// helpers the lanes still call for the u x u / y x y / d x d factorisations).  kw_lqr_* and kw_kf_* take no time range: a
+// large system always runs one segment.
+template <class DM, class T>
+struct Chunk {
+  static constexpr bool BIG = is_big<DM>();
+  static constexpr unsigned WTHR = 32 * BW_WARPS;   // threads per CTA of the warp-per-sample kernels
+  const Call& c;
+  const Plan& p;
+  char* base;               // this slice's part of the workspace
+  size_t s0;                // first sample of the chunk
+  int n, npad, nblk, wblk;  // samples (valid, padded to 32); CTAs of the thread- and of the warp-per-sample kernels
+  int Tn, N;
+  bool tv, vjp;
+  bool warp_cov;            // covariance kernels one warp per sample (always for the large systems)
+  size_t xcs = 0;           // element stride between the repacked observation sets in xc (repack_obs)
+
+  double* D(size_t off) const { return (double*)(base + off); }
+  float* F(size_t off) const { return (float*)(base + off); }
+  size_t tstride() const { return tv ? (size_t)DM::CL.total * p.Sc : 0; }
+  int rt() const { return trial_rt(N, trial_rt_max<DM>()); }
+
+  int pack(cudaStream_t st) const {
+    PackArgs<T> pa{};
+    pa.act = *c.act;
+    if (c.dyn) pa.dyn = *c.dyn;
+    pa.sigma0 = c.sigma0 ? *c.sigma0 : LqgkMat{nullptr, 0, 0};
+    pa.x = DM::X; pa.b = DM::B; pa.u = DM::U; pa.y = DM::Y; pa.nT = Tn; pa.has_dyn = c.dyn != nullptr;
+    ProfScope ps_(PK_PACK, st);
+    k_pack<T><<<dim3((npad + 127) / 128, tv ? Tn : 1), 128, 0, st>>>(pa, (int)s0, n, npad, D(p.cst), p.Sc, tstride(), tv ? Tn : 1);
+    LQGK_LAUNCH_CHECK();
+    return LQGK_OK;
+  }
+  // Riccati sweep, t down.  AFFINE (gains entry point): also l_t and H_t.  VJP: keeps S_t for the adjoint.
+  template <bool AFFINE>
+  int lqr_fwd(cudaStream_t st) const {
+    double *Sric = vjp ? D(p.Sric) : nullptr, *l = AFFINE ? D(p.l) : nullptr, *H = AFFINE ? D(p.H) : nullptr;
+    int rc;
+    if constexpr (BIG) {
+      const size_t smem = BigG<DM>::smem_lqr();
+      if ((rc = set_smem<DM>((const void*)kw_lqr_fwd<DM, AFFINE>, smem))) return rc;
+      ProfScope ps_(PK_LQR_FWD, st);
+      kw_lqr_fwd<DM, AFFINE><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, c.eps, D(p.L), vjp, Sric, l, H);
+      LQGK_LAUNCH_CHECK();
+    } else {
+      const size_t smem = sizeof(double) * 32 * (AFFINE ? LqrC<DM>::n_affine : LqrC<DM>::n);
+      if ((rc = set_smem<DM>((const void*)k_lqr_fwd<DM, AFFINE>, smem))) return rc;
+      ProfScope ps_(PK_LQR_FWD, st);
+      k_lqr_fwd<DM, AFFINE><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, c.eps, D(p.L), vjp, Sric, l, H);
+      LQGK_LAUNCH_CHECK();
+    }
+    return LQGK_OK;
+  }
+  // Kalman sweep, t up over [t0, t1).  VJP: keeps P_t for the adjoint.
+  int kf_fwd(cudaStream_t st, int t0, int t1) const {
+    double* Pkf = vjp ? D(p.Pkf) : nullptr;
+    int rc;
+    if constexpr (BIG) {
+      const size_t smem = BigG<DM>::smem_kf();
+      if ((rc = set_smem<DM>((const void*)kw_kf_fwd<DM>, smem))) return rc;
+      ProfScope ps_(PK_KF_FWD, st);
+      kw_kf_fwd<DM><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, D(p.K), vjp, Pkf);
+      LQGK_LAUNCH_CHECK();
+    } else {
+      const size_t smem = sizeof(double) * 32 * KfC<DM>::n;
+      if ((rc = set_smem<DM>((const void*)k_kf_fwd<DM>, smem))) return rc;
+      ProfScope ps_(PK_KF_FWD, st);
+      k_kf_fwd<DM><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, D(p.K), vjp, Pkf, t0, t1);
+      LQGK_LAUNCH_CHECK();
+    }
+    return LQGK_OK;
+  }
+  // Covariance pass, t up over [t0, t1): the per-trial records; VJP: also the adjoint's linearisation points.
+  int cov_fwd(cudaStream_t st, int t0, int t1) const {
+    double *Cs = vjp ? D(p.Cs) : nullptr, *J0 = vjp ? D(p.J0) : nullptr;
+    float *FU = vjp ? F(p.FU) : nullptr, *JS = vjp ? F(p.JS) : nullptr;
+    int rc;
+    if (warp_cov) {
+      const size_t smem = BigW<DM>::smem_fwd();
+      if ((rc = set_smem<DM>((const void*)kw_cov_fwd<DM, !BIG>, smem))) return rc;
+      ProfScope ps_(PK_COV_FWD, st);
+      kw_cov_fwd<DM, !BIG><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, D(p.L), D(p.K), vjp, Cs, FU, JS, J0, F(p.rec), t0, t1);
+      LQGK_LAUNCH_CHECK();
+    } else if constexpr (!BIG) {
+      const size_t smem = smem_cov_fwd<DM>();
+      if ((rc = set_smem<DM>((const void*)k_cov_fwd<DM>, smem))) return rc;
+      ProfScope ps_(PK_COV_FWD, st);
+      k_cov_fwd<DM><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, D(p.L), D(p.K), vjp, Cs, FU, JS, J0, F(p.rec), t0, t1);
+      LQGK_LAUNCH_CHECK();
+    }
+    return LQGK_OK;
+  }
+  // Observations of the chunk in the per-trial kernels' component-major layout (k_repack_obs): one data set shared by all
+  // samples (x_sample_stride == 0) or one per sample of the chunk.
+  int repack_obs(cudaStream_t st) {
+    const LqgkDims& d = *c.dims;
+    const int row = 32 * rt(), nb = (N + row - 1) / row;
+    const bool per_sample = d.x_sample_stride != 0;
+    const size_t per = (size_t)(Tn + 1) * nb * d.d * row;
+    const int nsets = per_sample ? n : 1;
+    xcs = per_sample ? per : 0;
+    const size_t total = per * nsets;
+    const unsigned blocks = (unsigned)std::min<size_t>((total + 255) / 256, (size_t)sm_count() * 16);
+    ProfScope ps_(PK_PACK, st);
+    k_repack_obs<float><<<blocks, 256, 0, st>>>(c.x_tm, (size_t)d.x_sample_stride, per_sample ? (int)s0 : 0, nsets, N, row, Tn + 1, d.d,
+                                                F(p.xc));
+    LQGK_LAUNCH_CHECK();
+    return LQGK_OK;
+  }
+  // Per-trial likelihood over the checkpoint segments [ka, kb).  VJP: stores the checkpoints of the carried state.
+  int trial_fwd(cudaStream_t st, int ka, int kb) const {
+    int rc = LQGK_E_UNSUPPORTED;
+    static_for<1, trial_rt_max<DM>() + 1>([&](auto RTC) {
+      if (rt() == decltype(RTC)::value)
+        rc = launch_trial_fwd<DM, decltype(RTC)::value>(st, F(p.rec), F(p.xc), xcs, n, N, Tn, D(p.ll), vjp ? F(p.hist) : nullptr, ka, kb);
+    });
+    return rc;
+  }
+  // Per-trial log-likelihoods out to the caller.  VJP: also the trial weights w (ll_bar; 1 without ll_bar and for the padded
+  // samples, whose results are never unpacked).
+  int store_ll(cudaStream_t st) const {
+    const size_t total = (size_t)n * N, padded = (size_t)npad * N;
+    ProfScope ps_(PK_MISC, st);
+    k_store_ll<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(p.ll), total, (T*)c.ll_out + s0 * N);
+    LQGK_LAUNCH_CHECK();
+    if (!vjp) return LQGK_OK;
+    auto load_w = [&](const T* ll_bar, size_t off, size_t count) -> int {
+      k_load_w<T><<<(unsigned)((count + 255) / 256), 256, 0, st>>>(ll_bar, count, F(p.w) + off);
+      LQGK_LAUNCH_CHECK();
+      return LQGK_OK;
+    };
+    int rc;
+    if ((rc = load_w(c.ll_bar ? (const T*)c.ll_bar + s0 * N : nullptr, 0, total))) return rc;
+    return padded > total ? load_w(nullptr, total, padded - total) : LQGK_OK;
+  }
+  // Zeroes the cotangent accumulators, and the per-step sums of the padded samples: k_trial_rev never writes those, and the
+  // covariance adjoint must read finite data.
+  int zero_acc(cudaStream_t st) const {
+    if (cudaMemsetAsync(D(p.acc), 0, sizeof(double) * DM::CL.total * p.Sc, st) != cudaSuccess) return LQGK_E_CUDA;
+    if (npad > n &&
+        cudaMemsetAsync(F(p.sums) + (size_t)n * Tn * DM::SUMP, 0, sizeof(float) * (size_t)(npad - n) * Tn * DM::SUMP, st) != cudaSuccess)
+      return LQGK_E_CUDA;
+    return LQGK_OK;
+  }
+  // Per-trial adjoint over the checkpoint segments [ka, kb), walked downwards: the per-step sums over trials.
+  int trial_rev(cudaStream_t st, int ka, int kb) const {
+    int rc = LQGK_E_UNSUPPORTED;
+    static_for<1, trial_rt_max<DM>() + 1>([&](auto RTC) {
+      if (rt() == decltype(RTC)::value)
+        rc = launch_trial_rev<DM, decltype(RTC)::value>(st, F(p.rec), F(p.xc), xcs, F(p.hist), F(p.w), n, N, Tn, F(p.sums), F(p.carcb), ka,
+                                                        kb);
+    });
+    return rc;
+  }
+  // Sequential covariance adjoint, t down over [t0, t1); carC hands its carry from one segment to the next.
+  int cov_seq_rev(cudaStream_t st, int t0, int t1) const {
+    int rc;
+    if (warp_cov) {
+      const size_t smem = BigW<DM>::smem_seq();
+      if ((rc = set_smem<DM>((const void*)kw_cov_seq_rev<DM>, smem))) return rc;
+      ProfScope ps_(PK_COV_REV, st);
+      kw_cov_seq_rev<DM><<<wblk, WTHR, smem, st>>>(npad, Tn, N, F(p.w), F(p.FU), F(p.JS), D(p.J0), F(p.sums), F(p.SGB), D(p.SGBI), F(p.SFW), t0,
+                                                   t1, D(p.carC));
+      LQGK_LAUNCH_CHECK();
+    } else if constexpr (!BIG) {
+      const size_t smem = smem_cov_seq_rev<DM>();
+      if ((rc = set_smem<DM>((const void*)k_cov_seq_rev<DM>, smem))) return rc;
+      ProfScope ps_(PK_COV_REV, st);
+      k_cov_seq_rev<DM><<<nblk, 32, smem, st>>>(p.Sc, Tn, N, F(p.w), F(p.FU), F(p.JS), D(p.J0), F(p.sums), F(p.SGB), D(p.SGBI), F(p.SFW), t0, t1,
+                                                D(p.carC));
+      LQGK_LAUNCH_CHECK();
+    }
+    return LQGK_OK;
+  }
+  // Time-parallel contraction of the adjoint over [t0, t1), cut into grid.y time ranges: the cotangent accumulators, Lbar, Kbar.
+  int contraction(cudaStream_t st, int t0, int t1) const {
+    const int len = t1 - t0;
+    int rc;
+    ProfScope ps_(PK_COV_CONTRIB, st);
+    if (warp_cov) {
+      // enough (sample x range) warps to put ~12 on every SM when there are few samples
+      const int chunks = std::max(1, std::min((len + 3) / 4, (sm_count() * 12 + npad - 1) / npad));
+      const size_t smem = BigW<DM>::smem_con();
+      if ((rc = set_smem<DM>((const void*)kw_cov_contrib<DM, !BIG>, smem))) return rc;
+      kw_cov_contrib<DM, !BIG><<<dim3(wblk, chunks), WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI),
+                                                                      F(p.SFW), F(p.sums), D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), t0, t1);
+      LQGK_LAUNCH_CHECK();
+    } else if constexpr (!BIG) {
+      // (sample-group x time-range) warps: enough to occupy every SM a few times over
+      const int cwarps = g_contrib_warps > 0 ? g_contrib_warps : sm_count() * 30;
+      const dim3 grid(nblk, std::max(1, std::min((len + 7) / 8, (cwarps + nblk - 1) / nblk)));
+      auto pass = [&](auto P) -> int {
+        constexpr int PASS = decltype(P)::value;
+        const size_t smem = smem_cov_contrib<DM, PASS>();
+        if (int rcs = set_smem<DM>((const void*)k_cov_contrib<DM, PASS>, smem)) return rcs;
+        k_cov_contrib<DM, PASS><<<grid, 32, smem, st>>>(D(p.cst), p.Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW), F(p.sums),
+                                                        D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), t0, t1);
+        LQGK_LAUNCH_CHECK();
+        return LQGK_OK;
+      };
+      if constexpr (contrib_merged<DM>()) return pass(std::integral_constant<int, 2>{});   // both passes in one kernel
+      else if ((rc = pass(std::integral_constant<int, 0>{}))) return rc;
+      else return pass(std::integral_constant<int, 1>{});
+    }
+    return LQGK_OK;
+  }
+  // Kalman-gain adjoint, t down over [t0, t1); carP hands its carry from one segment to the next.
+  int kf_rev(cudaStream_t st, int t0, int t1) const {
+    int rc;
+    if constexpr (BIG) {
+      const size_t smem = BigG<DM>::smem_kf();
+      if ((rc = set_smem<DM>((const void*)kw_kf_rev<DM>, smem))) return rc;
+      ProfScope ps_(PK_KF_REV, st);
+      kw_kf_rev<DM><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, D(p.Pkf), D(p.Kbar), D(p.acc));
+      LQGK_LAUNCH_CHECK();
+    } else {
+      const size_t smem = smem_kf_rev<DM>();
+      if ((rc = set_smem<DM>((const void*)k_kf_rev<DM>, smem))) return rc;
+      ProfScope ps_(PK_KF_REV, st);
+      k_kf_rev<DM><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, Tn, D(p.Pkf), D(p.Kbar), D(p.KbarF), D(p.acc), t0, t1, D(p.carP));
+      LQGK_LAUNCH_CHECK();
+    }
+    return LQGK_OK;
+  }
+  // Riccati adjoint, t up; needs Lbar complete.
+  int lqr_rev(cudaStream_t st) const {
+    int rc;
+    if constexpr (BIG) {
+      const size_t smem = BigG<DM>::smem_lqr();
+      if ((rc = set_smem<DM>((const void*)kw_lqr_rev<DM>, smem))) return rc;
+      ProfScope ps_(PK_LQR_REV, st);
+      kw_lqr_rev<DM><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, c.eps, D(p.L), D(p.Sric), D(p.Lbar), D(p.acc));
+      LQGK_LAUNCH_CHECK();
+    } else {
+      const size_t smem = smem_lqr_rev<DM>();
+      if ((rc = set_smem<DM>((const void*)k_lqr_rev<DM>, smem))) return rc;
+      ProfScope ps_(PK_LQR_REV, st);
+      k_lqr_rev<DM><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, Tn, c.eps, D(p.L), D(p.Sric), D(p.Lbar), D(p.acc));
+      LQGK_LAUNCH_CHECK();
+    }
+    return LQGK_OK;
+  }
+  // Cotangent accumulators -> the caller's gradient structs.
+  int unpack(cudaStream_t st) const {
+    UnpackArgs<T> ua{};
+    ua.act = *c.act; ua.dyn = *c.dyn; ua.sigma0 = c.sigma0 ? *c.sigma0 : LqgkMat{nullptr, 0, 0};
+    if (c.gact) ua.gact = *c.gact;
+    if (c.gdyn) ua.gdyn = *c.gdyn;
+    if (c.gsig0) ua.gsigma0 = *c.gsig0;
+    ua.x = DM::X; ua.b = DM::B; ua.u = DM::U; ua.y = DM::Y;
+    ProfScope ps_(PK_UNPACK, st);
+    k_unpack<T><<<(n + 63) / 64, 64, 0, st>>>(ua, (int)s0, n, D(p.acc), D(p.cst), p.Sc);
+    LQGK_LAUNCH_CHECK();
+    return LQGK_OK;
+  }
+  // Gains [t][E] per sample out to the caller: a transposing copy of the sample-minor workspace arrays of the small systems,
+  // a plain copy of the sample-major ones of the large systems.
+  int store_gains(cudaStream_t st, size_t off, int E, void* out) const {
+    if (!out) return LQGK_OK;
+    const size_t total = (size_t)n * Tn * E;
+    if constexpr (BIG)
+      k_store_ll<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(off), total, (T*)out + s0 * Tn * E);
+    else
+      k_store_rows<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(off), p.Sc, n, Tn, E, (T*)out + s0 * Tn * E);
+    LQGK_LAUNCH_CHECK();
+    return LQGK_OK;
+  }
+  // Full predictive moments (conditional_moments / belief_tracking_distribution), small systems only: thread-per-sample
+  // covariance kernel writing Sigma in the caller's layout, thread-per-trial mean kernel.
+  int moments(cudaStream_t st) const {
+    if constexpr (BIG) {
+      return LQGK_E_UNSUPPORTED;
+    } else {
+      {
+        size_t smem = sizeof(double) * 32 * CovC<DM>::n;
+        ProfScope ps_(PK_COV_FWD, st);
+        k_cov_moments<DM, T><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, n, D(p.L), D(p.K), F(p.rec),
+                                                     c.Sig_out ? (T*)c.Sig_out + s0 * Tn * DM::N * DM::N : nullptr);
+        LQGK_LAUNCH_CHECK();
+      }
+      if (c.mu_out) {
+        size_t total = (size_t)n * N;
+        ProfScope ps_(PK_TRIAL_FWD, st);
+        k_trial_moments<DM, T><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(F(p.rec), c.x_tm, (size_t)c.dims->x_sample_stride, (int)s0, n,
+                                                                              N, Tn, (T*)c.mu_out + s0 * N * Tn * DM::N);
+        LQGK_LAUNCH_CHECK();
+      }
+      return LQGK_OK;
+    }
+  }
+};
+
 template <class DM, class T>
 int run(const Call& c) {
   const LqgkDims& d = *c.dims;
-  constexpr CLayout cl = DM::CL;
   const bool has_dyn = c.dyn != nullptr;
   const bool tv = spec_time_varying(*c.act, true) || (has_dyn && spec_time_varying(*c.dyn, false));
   if (tv && c.mode == LQGK_MODE_VJP) return LQGK_E_UNSUPPORTED;
+  // large systems: no time-varying specs, and the predictive moments stay on the host-side slow path
+  if (is_big<DM>() && (tv || c.mode == LQGK_MODE_MOMENTS)) return LQGK_E_UNSUPPORTED;
   if (!c.ws || ((uintptr_t)c.ws % ALIGN) != 0) return LQGK_E_INVALID;
   // slices: ns concurrent streams, each with its own workspace part and chunk size Sc
   int ns = c.mode == LQGK_MODE_GAINS ? 1 : std::max(1, std::min(g_streams, (int)((d.S + 31) / 32)));
@@ -319,13 +615,15 @@ int run(const Call& c) {
   if (Sc == 0) return LQGK_E_WORKSPACE;
   const Plan p = make_plan<DM>(d, c.mode, tv, Sc);
   const size_t slice_bytes = up(p.bytes, ALIGN);
-  char* base = (char*)c.ws;
-  auto D = [&](size_t off) { return (double*)(base + off); };
-  auto F = [&](size_t off) { return (float*)(base + off); };
-  cudaStream_t st = c.stream;
-  const int auxm = c.mode == LQGK_MODE_VJP ? g_aux_streams : 0;
-  const bool aux = auxm != 0;
-  const int nstreams = (ns > 1 ? ns : 0) + (aux ? 3 * ns : 0);
+  const int Tn = d.T, N = d.N;
+  const bool vjp = c.mode == LQGK_MODE_VJP;
+  // time segments of the launch sequence of a chunk of n samples (see below)
+  auto segments = [&](int n) {
+    if (is_big<DM>() || !vjp || g_aux_streams == 0 || n > g_pipe_max_samples) return 1;
+    return std::max(1, std::min(g_pipe_segments, trial_geom<DM>(N, Tn).nseg));
+  };
+  const bool pipelined = segments((int)((size_t)d.S - ((size_t)d.S - 1) / Sc * Sc)) > 1;   // (the last chunk is the smallest)
+  const int nstreams = (ns > 1 ? ns : 0) + (pipelined ? 3 * ns : 0);
   if (nstreams > 0) {
     if (int rcp = g_pool.acquire(nstreams, c.stream)) return rcp;
   }
@@ -372,425 +670,87 @@ int run(const Call& c) {
       }
     }
   } joiner{nstreams, c.stream, &touched};
-  const int Tn = d.T, N = d.N;
-  const size_t tstride = tv ? (size_t)cl.total * Sc : 0;
-
-  PackArgs<T> pa{};
-  pa.act = *c.act;
-  if (has_dyn) pa.dyn = *c.dyn;
-  pa.sigma0 = c.sigma0 ? *c.sigma0 : LqgkMat{nullptr, 0, 0};
-  pa.x = DM::X; pa.b = DM::B; pa.u = DM::U; pa.y = DM::Y; pa.nT = Tn; pa.has_dyn = has_dyn;
 
   int chunk_idx = 0;
   for (size_t s0 = 0; s0 < (size_t)d.S; s0 += Sc, ++chunk_idx) {
     const int n = (int)std::min(Sc, (size_t)d.S - s0);
     const int npad = (int)up(n, 32);
-    const int nblk = npad / 32;
+    cudaStream_t st = c.stream;
+    char* base = (char*)c.ws;
     if (ns > 1) {
       st = g_pool.streams[chunk_idx % ns];
-      base = (char*)c.ws + (size_t)(chunk_idx % ns) * slice_bytes;
+      base += (size_t)(chunk_idx % ns) * slice_bytes;
     }
-    // auxiliary streams of this slice: independent kernels of one chunk run concurrently (they are latency-bound)
-    cudaStream_t x1 = aux ? g_pool.streams[aux0 + 3 * (chunk_idx % ns)] : st;
-    cudaStream_t x2 = aux ? g_pool.streams[aux0 + 3 * (chunk_idx % ns) + 1] : st;
-    cudaStream_t x3 = aux ? g_pool.streams[aux0 + 3 * (chunk_idx % ns) + 2] : st;
-    cudaStream_t a1 = (auxm & 1) ? x1 : st, a2 = st;
-    {
-      dim3 grid((npad + 127) / 128, tv ? Tn : 1);
-      ProfScope ps_(PK_PACK, st);
-      k_pack<T><<<grid, 128, 0, st>>>(pa, (int)s0, n, npad, D(p.cst), Sc, tstride, tv ? Tn : 1);
-      LQGK_LAUNCH_CHECK();
-    }
+    const bool warp_cov = is_big<DM>() || (!tv && d.S <= g_warp_cov_max_samples);
+    Chunk<DM, T> k{c, p, base, s0, n, npad, npad / 32, (npad + BW_WARPS - 1) / BW_WARPS, Tn, N, tv, vjp, warp_cov};
+    int rc;
+    if ((rc = k.pack(st))) return rc;
     if (c.mode == LQGK_MODE_GAINS) {
       if (c.L_out) {
-        size_t smem = sizeof(double) * 32 * LqrC<DM>::n_affine;
-        ProfScope ps_(PK_LQR_FWD, st);
-        k_lqr_fwd<DM, true><<<nblk, 32, smem, st>>>(D(p.cst), Sc, tstride, Tn, c.eps, D(p.L), 0, nullptr, D(p.l), D(p.H));
-        LQGK_LAUNCH_CHECK();
-        auto store = [&](size_t off, int E, void* out) -> int {
-          if (!out) return LQGK_OK;
-          size_t total = (size_t)n * Tn * E;
-          k_store_rows<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(off), Sc, n, Tn, E, (T*)out + s0 * Tn * E);
-          LQGK_LAUNCH_CHECK();
-          return LQGK_OK;
-        };
-        int rc;
-        if ((rc = store(p.L, DM::EL, c.L_out))) return rc;
-        if ((rc = store(p.l, DM::U, c.l_out))) return rc;
-        if ((rc = store(p.H, DM::U * DM::U, c.H_out))) return rc;
+        if ((rc = k.template lqr_fwd<true>(st))) return rc;
+        if ((rc = k.store_gains(st, p.L, DM::EL, c.L_out))) return rc;
+        if ((rc = k.store_gains(st, p.l, DM::U, c.l_out))) return rc;
+        if ((rc = k.store_gains(st, p.H, DM::U * DM::U, c.H_out))) return rc;
       }
       if (c.K_out) {
-        size_t smem = sizeof(double) * 32 * KfC<DM>::n;
-        ProfScope ps_(PK_KF_FWD, st);
-        k_kf_fwd<DM><<<nblk, 32, smem, st>>>(D(p.cst), Sc, tstride, Tn, D(p.K), 0, nullptr, 0, Tn);
-        LQGK_LAUNCH_CHECK();
-        size_t total = (size_t)n * Tn * DM::EK;
-        k_store_rows<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(p.K), Sc, n, Tn, DM::EK, (T*)c.K_out + s0 * Tn * DM::EK);
-        LQGK_LAUNCH_CHECK();
+        if ((rc = k.kf_fwd(st, 0, Tn))) return rc;
+        if ((rc = k.store_gains(st, p.K, DM::EK, c.K_out))) return rc;
       }
       continue;
     }
-    const bool vjp = c.mode == LQGK_MODE_VJP;
-    int rc;
-    const TrialGeom tgm = trial_geom<DM>(N, Tn);
-    const int G = (vjp && aux && !tv && n <= g_pipe_max_samples) ? std::max(1, std::min(g_pipe_segments, tgm.nseg)) : 1;
-    if (G > 1) {
-      // ---------------------------------------------------------------------------------------- pipelined launch sequence
-      // Few samples: every sweep over time is latency-bound (T dependent steps, ~1-2.5 ms each whatever the sample count) and the
-      // GPU idles behind the chain of nine sweeps.  The sweeps of one direction are therefore cut into G time segments and run as
-      // a software pipeline over internal streams: segment g of a consumer starts as soon as segment g of its producer is done.
-      //   t up  : kf_fwd (x1) -> cov_fwd (x2) -> trial_fwd (st)        [after lqr_fwd, which runs t down and feeds cov_fwd]
-      //   t down: trial_rev (st) -> cov_seq_rev (x1) -> contraction (x2) -> kf_rev (x3);  lqr_rev (t up) follows on x2
-      // Carries between segments: P_t, C_t and the checkpoints of c_t are stored per step anyway (adjoint linearisation points);
-      // the adjoint carries (cb, Cb, Pnb) go through three small buffers.
-      const bool warp_cov_p = d.S <= g_warp_cov_max_samples;
-      const int wblk_p = (npad + BW_WARPS - 1) / BW_WARPS;
-      const int RTp = tgm.RT;
-      std::vector<int> kb(G + 1), tb(G + 1);
-      for (int g = 0; g <= G; ++g) { kb[g] = (int)((long long)g * tgm.nseg / G); tb[g] = std::min(Tn, kb[g] * tgm.CK); }
-      dep(st, x1);                                 // pack done -> kf_fwd on x1 beside lqr_fwd on st
-      {
-        size_t smem = sizeof(double) * 32 * LqrC<DM>::n;
-        ProfScope ps_(PK_LQR_FWD, st);
-        k_lqr_fwd<DM, false><<<nblk, 32, smem, st>>>(D(p.cst), Sc, tstride, Tn, c.eps, D(p.L), 1, D(p.Sric), nullptr, nullptr);
-        LQGK_LAUNCH_CHECK();
-      }
-      dep(st, x2);                                 // L complete -> covariance pass
-      size_t xcs = 0;
-      if ((rc = launch_repack_obs(st, d, 32 * RTp, c.x_tm, (int)s0, n, F(p.xc), &xcs))) return rc;
-      const size_t sm_kf = sizeof(double) * 32 * KfC<DM>::n;
-      const size_t sm_cov = warp_cov_p ? BigW<DM>::smem_fwd() : smem_cov_fwd<DM>();
-      if (warp_cov_p) { if ((rc = set_smem<DM>((const void*)kw_cov_fwd<DM, true>, sm_cov))) return rc; }
-      else { if ((rc = set_smem<DM>((const void*)k_cov_fwd<DM>, sm_cov))) return rc; }
-      for (int g = 0; g < G; ++g) {
-        {
-          ProfScope ps_(PK_KF_FWD, x1);
-          k_kf_fwd<DM><<<nblk, 32, sm_kf, x1>>>(D(p.cst), Sc, tstride, Tn, D(p.K), 1, D(p.Pkf), tb[g], tb[g + 1]);
-          LQGK_LAUNCH_CHECK();
-        }
-        dep(x1, x2);
-        {
-          ProfScope ps_(PK_COV_FWD, x2);
-          if (warp_cov_p)
-            kw_cov_fwd<DM, true><<<wblk_p, 32 * BW_WARPS, sm_cov, x2>>>(D(p.cst), Sc, npad, Tn, D(p.L), D(p.K), 1, D(p.Cs), F(p.FU), F(p.JS), D(p.J0),
-                                                                        F(p.rec), tb[g], tb[g + 1]);
-          else
-            k_cov_fwd<DM><<<nblk, 32, sm_cov, x2>>>(D(p.cst), Sc, tstride, Tn, D(p.L), D(p.K), 1, D(p.Cs), F(p.FU), F(p.JS), D(p.J0), F(p.rec),
-                                                    tb[g], tb[g + 1]);
-          LQGK_LAUNCH_CHECK();
-        }
-        dep(x2, st);
-        rc = LQGK_E_UNSUPPORTED;
-        static_for<1, trial_rt_max<DM>() + 1>([&](auto RTC) {
-          if (RTp == decltype(RTC)::value)
-            rc = launch_trial_fwd<DM, decltype(RTC)::value>(st, F(p.rec), F(p.xc), xcs, n, N, Tn, D(p.ll), F(p.hist), kb[g], kb[g + 1]);
-        });
-        if (rc) return rc;
-      }
-      {
-        size_t total = (size_t)n * N;
-        ProfScope ps_(PK_MISC, st);
-        k_store_ll<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(p.ll), total, (T*)c.ll_out + s0 * N);
-        LQGK_LAUNCH_CHECK();
-        size_t totalp = (size_t)npad * N;
-        const T* lb = c.ll_bar ? (const T*)c.ll_bar + s0 * N : nullptr;
-        k_load_w<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(lb, total, F(p.w));
-        LQGK_LAUNCH_CHECK();
-        if (totalp > total) {
-          k_load_w<T><<<(unsigned)((totalp - total + 255) / 256), 256, 0, st>>>(nullptr, totalp - total, F(p.w) + total);
-          LQGK_LAUNCH_CHECK();
-        }
-      }
-      if (cudaMemsetAsync(D(p.acc), 0, sizeof(double) * cl.total * Sc, st) != cudaSuccess) return LQGK_E_CUDA;
-      if (npad > n) {
-        if (cudaMemsetAsync(F(p.sums) + (size_t)n * Tn * DM::SUMP, 0, sizeof(float) * (size_t)(npad - n) * Tn * DM::SUMP, st) != cudaSuccess)
-          return LQGK_E_CUDA;
-      }
-      const size_t sm_seq = warp_cov_p ? BigW<DM>::smem_seq() : smem_cov_seq_rev<DM>();
-      const size_t sm_con = warp_cov_p ? BigW<DM>::smem_con() : 0;
-      if (warp_cov_p) {
-        if ((rc = set_smem<DM>((const void*)kw_cov_seq_rev<DM>, sm_seq))) return rc;
-        if ((rc = set_smem<DM>((const void*)kw_cov_contrib<DM, true>, sm_con))) return rc;
-      } else {
-        if ((rc = set_smem<DM>((const void*)k_cov_seq_rev<DM>, sm_seq))) return rc;
-      }
-      const size_t sm_kfr = smem_kf_rev<DM>();
-      if ((rc = set_smem<DM>((const void*)k_kf_rev<DM>, sm_kfr))) return rc;
-      for (int g = G - 1; g >= 0; --g) {
-        rc = LQGK_E_UNSUPPORTED;
-        static_for<1, trial_rt_max<DM>() + 1>([&](auto RTC) {
-          if (RTp == decltype(RTC)::value)
-            rc = launch_trial_rev<DM, decltype(RTC)::value>(st, F(p.rec), F(p.xc), xcs, F(p.hist), F(p.w), n, N, Tn, F(p.sums), F(p.carcb), kb[g],
-                                                            kb[g + 1]);
-        });
-        if (rc) return rc;
-        dep(st, x1);
-        {
-          ProfScope ps_(PK_COV_REV, x1);
-          if (warp_cov_p)
-            kw_cov_seq_rev<DM><<<wblk_p, 32 * BW_WARPS, sm_seq, x1>>>(npad, Tn, N, F(p.w), F(p.FU), F(p.JS), D(p.J0), F(p.sums), F(p.SGB), D(p.SGBI),
-                                                                     F(p.SFW), tb[g], tb[g + 1], D(p.carC));
-          else
-            k_cov_seq_rev<DM><<<nblk, 32, sm_seq, x1>>>(Sc, Tn, N, F(p.w), F(p.FU), F(p.JS), D(p.J0), F(p.sums), F(p.SGB), D(p.SGBI), F(p.SFW), tb[g],
-                                                        tb[g + 1], D(p.carC));
-          LQGK_LAUNCH_CHECK();
-        }
-        dep(x1, x2);
-        {
-          const int len = tb[g + 1] - tb[g];
-          ProfScope ps_(PK_COV_CONTRIB, x2);
-          if (warp_cov_p) {
-            int chunks = std::max(1, std::min((len + 3) / 4, (sm_count() * 12 + npad - 1) / npad));   // (segments run one after the other)
-            kw_cov_contrib<DM, true><<<dim3(wblk_p, chunks), 32 * BW_WARPS, sm_con, x2>>>(D(p.cst), Sc, npad, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB),
-                                                                                       D(p.SGBI), F(p.SFW), F(p.sums), D(p.acc), D(p.Lbar),
-                                                                                       D(p.Kbar), D(p.KbarF), tb[g], tb[g + 1]);
-            LQGK_LAUNCH_CHECK();
-          } else {
-            const int cwarps = g_contrib_warps > 0 ? g_contrib_warps : sm_count() * 30;
-            int chunks = std::max(1, std::min((len + 7) / 8, (cwarps + nblk - 1) / nblk));
-            dim3 grid(nblk, chunks);
-            if constexpr (contrib_merged<DM>()) {
-              size_t smem = smem_cov_contrib<DM, 2>();
-              if ((rc = set_smem<DM>((const void*)k_cov_contrib<DM, 2>, smem))) return rc;
-              k_cov_contrib<DM, 2><<<grid, 32, smem, x2>>>(D(p.cst), Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW), F(p.sums),
-                                                          D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), tb[g], tb[g + 1]);
-              LQGK_LAUNCH_CHECK();
-            } else {
-              size_t smem0 = smem_cov_contrib<DM, 0>(), smem1 = smem_cov_contrib<DM, 1>();
-              if ((rc = set_smem<DM>((const void*)k_cov_contrib<DM, 0>, smem0))) return rc;
-              if ((rc = set_smem<DM>((const void*)k_cov_contrib<DM, 1>, smem1))) return rc;
-              k_cov_contrib<DM, 0><<<grid, 32, smem0, x2>>>(D(p.cst), Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW), F(p.sums),
-                                                           D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), tb[g], tb[g + 1]);
-              LQGK_LAUNCH_CHECK();
-              k_cov_contrib<DM, 1><<<grid, 32, smem1, x2>>>(D(p.cst), Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW), F(p.sums),
-                                                           D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), tb[g], tb[g + 1]);
-              LQGK_LAUNCH_CHECK();
-            }
-          }
-        }
-        dep(x2, x3);
-        {
-          ProfScope ps_(PK_KF_REV, x3);
-          k_kf_rev<DM><<<nblk, 32, sm_kfr, x3>>>(D(p.cst), Sc, Tn, D(p.Pkf), D(p.Kbar), D(p.KbarF), D(p.acc), tb[g], tb[g + 1], D(p.carP));
-          LQGK_LAUNCH_CHECK();
-        }
-      }
-      {
-        size_t smem = smem_lqr_rev<DM>();
-        if ((rc = set_smem<DM>((const void*)k_lqr_rev<DM>, smem))) return rc;
-        ProfScope ps_(PK_LQR_REV, x2);            // after every contraction segment (Lbar complete), in order on x2
-        k_lqr_rev<DM><<<nblk, 32, smem, x2>>>(D(p.cst), Sc, Tn, c.eps, D(p.L), D(p.Sric), D(p.Lbar), D(p.acc));
-        LQGK_LAUNCH_CHECK();
-      }
-      dep(x2, st);
-      dep(x3, st);
-      {
-        UnpackArgs<T> ua{};
-        ua.act = *c.act; ua.dyn = *c.dyn; ua.sigma0 = pa.sigma0;
-        if (c.gact) ua.gact = *c.gact;
-        if (c.gdyn) ua.gdyn = *c.gdyn;
-        if (c.gsig0) ua.gsigma0 = *c.gsig0;
-        ua.x = DM::X; ua.b = DM::B; ua.u = DM::U; ua.y = DM::Y;
-        ProfScope ps_(PK_UNPACK, st);
-        k_unpack<T><<<(n + 63) / 64, 64, 0, st>>>(ua, (int)s0, n, D(p.acc), D(p.cst), Sc);
-        LQGK_LAUNCH_CHECK();
-      }
-      continue;
-    }
-    dep(st, a1);                                   // pack done -> kf_fwd (a1) may run beside lqr_fwd (st)
-    {
-      size_t smem = sizeof(double) * 32 * LqrC<DM>::n;
-      ProfScope ps_(PK_LQR_FWD, st);
-      k_lqr_fwd<DM, false><<<nblk, 32, smem, st>>>(D(p.cst), Sc, tstride, Tn, c.eps, D(p.L), vjp, vjp ? D(p.Sric) : nullptr, nullptr, nullptr);
-      LQGK_LAUNCH_CHECK();
-    }
-    {
-      size_t smem = sizeof(double) * 32 * KfC<DM>::n;
-      ProfScope ps_(PK_KF_FWD, a1);
-      k_kf_fwd<DM><<<nblk, 32, smem, a1>>>(D(p.cst), Sc, tstride, Tn, D(p.K), vjp, vjp ? D(p.Pkf) : nullptr, 0, Tn);
-      LQGK_LAUNCH_CHECK();
-    }
-    dep(a1, st);
-    // Few samples (a handful of conditions, a few hundred chains per GPU): the thread-per-sample covariance kernels leave the
-    // GPU idle and every step costs one thread's instruction stream; the warp-per-sample kernels of the large systems spread
-    // a step over 32 lanes (S = 8: covariance forward 3.3 -> 2.4 ms, sequential adjoint 2.5 -> 1.0 ms) and win up to ~1,000
-    // samples.  The Riccati / Kalman sweeps stay thread-per-sample (3 x 3 products do not spread), hence GAINS_MINOR.
     if (c.mode == LQGK_MODE_MOMENTS) {
-      // slow path: full predictive moments (conditional_moments / belief_tracking_distribution), thread-per-sample covariance
-      // kernel writing Sigma in the caller's layout, thread-per-trial mean kernel
-      {
-        size_t smem = sizeof(double) * 32 * CovC<DM>::n;
-        ProfScope ps_(PK_COV_FWD, st);
-        k_cov_moments<DM, T><<<nblk, 32, smem, st>>>(D(p.cst), Sc, tstride, Tn, n, D(p.L), D(p.K), F(p.rec),
-                                                     c.Sig_out ? (T*)c.Sig_out + s0 * Tn * DM::N * DM::N : nullptr);
-        LQGK_LAUNCH_CHECK();
-      }
-      if (c.mu_out) {
-        size_t total = (size_t)n * N;
-        ProfScope ps_(PK_TRIAL_FWD, st);
-        k_trial_moments<DM, T><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(F(p.rec), c.x_tm, (size_t)d.x_sample_stride, (int)s0, n, N, Tn,
-                                                                              (T*)c.mu_out + s0 * N * Tn * DM::N);
-        LQGK_LAUNCH_CHECK();
-      }
+      if ((rc = k.template lqr_fwd<false>(st))) return rc;
+      if ((rc = k.kf_fwd(st, 0, Tn))) return rc;
+      if ((rc = k.moments(st))) return rc;
       continue;
     }
-    const bool warp_cov = !tv && d.S <= g_warp_cov_max_samples;
-    const int wblk = (npad + BW_WARPS - 1) / BW_WARPS;
-    if (warp_cov) {
-      size_t smem = BigW<DM>::smem_fwd();
-      if ((rc = set_smem<DM>((const void*)kw_cov_fwd<DM, true>, smem))) return rc;
-      ProfScope ps_(PK_COV_FWD, st);
-      kw_cov_fwd<DM, true><<<wblk, 32 * BW_WARPS, smem, st>>>(D(p.cst), Sc, npad, Tn, D(p.L), D(p.K), vjp, vjp ? D(p.Cs) : nullptr,
-                                                              vjp ? F(p.FU) : nullptr, vjp ? F(p.JS) : nullptr, vjp ? D(p.J0) : nullptr, F(p.rec));
-      LQGK_LAUNCH_CHECK();
-    } else {
-      size_t smem = smem_cov_fwd<DM>();
-      if ((rc = set_smem<DM>((const void*)k_cov_fwd<DM>, smem))) return rc;
-      ProfScope ps_(PK_COV_FWD, st);
-      k_cov_fwd<DM><<<nblk, 32, smem, st>>>(D(p.cst), Sc, tstride, Tn, D(p.L), D(p.K), vjp, vjp ? D(p.Cs) : nullptr, vjp ? F(p.FU) : nullptr,
-                                            vjp ? F(p.JS) : nullptr, vjp ? D(p.J0) : nullptr, F(p.rec), 0, Tn);
-      LQGK_LAUNCH_CHECK();
+    // Launch sequence of the likelihood and its adjoint.  Few samples: every sweep over time is latency-bound (T dependent
+    // steps, ~1-2.5 ms each whatever the sample count) and the GPU idles behind the chain of nine sweeps.  The sweeps of one
+    // direction are therefore cut into G time segments and run as a software pipeline over the chunk's internal streams
+    // x1..x3: segment g of a consumer starts as soon as segment g of its producer is done.
+    //   t up  : kf_fwd (x1) -> cov_fwd (x2) -> trial_fwd (st)        [after lqr_fwd, which runs t down and feeds cov_fwd]
+    //   t down: trial_rev (st) -> cov_seq_rev (x1) -> contraction (x2) -> kf_rev (x3);  lqr_rev (t up) follows on x2
+    // Carries between segments: P_t, C_t and the checkpoints of c_t are stored per step anyway (adjoint linearisation points);
+    // the adjoint carries (cb, Cb, Pnb) go through three small buffers.  G = 1 (forward only, large systems, kernel overlap
+    // off, chunks above g_pipe_max_samples, T within one checkpoint interval) is the same sequence on the chunk's stream.
+    const int G = segments(n);
+    cudaStream_t x1 = st, x2 = st, x3 = st;
+    if (G > 1) {
+      const int a = aux0 + 3 * (chunk_idx % ns);
+      x1 = g_pool.streams[a];
+      x2 = g_pool.streams[a + 1];
+      x3 = g_pool.streams[a + 2];
     }
-    const int RT = std::min((N + 31) / 32, trial_rt_max<DM>());
-    float* hist = vjp ? F(p.hist) : nullptr;
-    size_t xcs = 0;
-    if ((rc = launch_repack_obs(st, d, 32 * RT, c.x_tm, (int)s0, n, F(p.xc), &xcs))) return rc;
-    rc = LQGK_E_UNSUPPORTED;
-    static_for<1, trial_rt_max<DM>() + 1>([&](auto RTC) {
-      if (RT == decltype(RTC)::value) rc = launch_trial_fwd<DM, decltype(RTC)::value>(st, F(p.rec), F(p.xc), xcs, n, N, Tn, D(p.ll), hist);
-    });
-    if (rc) return rc;
-    {
-      size_t total = (size_t)n * N;
-      ProfScope ps_(PK_MISC, st);
-      k_store_ll<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(D(p.ll), total, (T*)c.ll_out + s0 * N);
-      LQGK_LAUNCH_CHECK();
+    const TrialGeom tg = trial_geom<DM>(N, Tn);
+    std::vector<int> kb(G + 1), tb(G + 1);   // segment g: checkpoint segments [kb[g], kb[g + 1]), steps [tb[g], tb[g + 1])
+    for (int g = 0; g <= G; ++g) { kb[g] = (int)((long long)g * tg.nseg / G); tb[g] = std::min(Tn, kb[g] * tg.CK); }
+    dep(st, x1);                                 // pack done -> kf_fwd on x1 beside lqr_fwd on st
+    if ((rc = k.template lqr_fwd<false>(st))) return rc;
+    dep(st, x2);                                 // L complete -> covariance pass
+    if ((rc = k.repack_obs(st))) return rc;
+    for (int g = 0; g < G; ++g) {
+      if ((rc = k.kf_fwd(x1, tb[g], tb[g + 1]))) return rc;
+      dep(x1, x2);
+      if ((rc = k.cov_fwd(x2, tb[g], tb[g + 1]))) return rc;
+      dep(x2, st);
+      if ((rc = k.trial_fwd(st, kb[g], kb[g + 1]))) return rc;
     }
+    if ((rc = k.store_ll(st))) return rc;
     if (!vjp) continue;
-    {
-      size_t total = (size_t)npad * N;   // padded samples get weight of... the same trials; harmless (never unpacked)
-      const T* lb = c.ll_bar ? (const T*)c.ll_bar + s0 * N : nullptr;
-      size_t valid = (size_t)n * N;
-      k_load_w<T><<<(unsigned)((valid + 255) / 256), 256, 0, st>>>(lb, valid, F(p.w));
-      LQGK_LAUNCH_CHECK();
-      if (total > valid) {
-        k_load_w<T><<<(unsigned)((total - valid + 255) / 256), 256, 0, st>>>(nullptr, total - valid, F(p.w) + valid);
-        LQGK_LAUNCH_CHECK();
-      }
+    if ((rc = k.zero_acc(st))) return rc;
+    for (int g = G - 1; g >= 0; --g) {
+      if ((rc = k.trial_rev(st, kb[g], kb[g + 1]))) return rc;
+      dep(st, x1);
+      if ((rc = k.cov_seq_rev(x1, tb[g], tb[g + 1]))) return rc;
+      dep(x1, x2);
+      if ((rc = k.contraction(x2, tb[g], tb[g + 1]))) return rc;
+      dep(x2, x3);
+      if ((rc = k.kf_rev(x3, tb[g], tb[g + 1]))) return rc;
     }
-    rc = LQGK_E_UNSUPPORTED;
-    static_for<1, trial_rt_max<DM>() + 1>([&](auto RTC) {
-      if (RT == decltype(RTC)::value)
-        rc = launch_trial_rev<DM, decltype(RTC)::value>(st, F(p.rec), F(p.xc), xcs, hist, F(p.w), n, N, Tn, F(p.sums), F(p.carcb));
-    });
-    if (rc) return rc;
-    if (cudaMemsetAsync(D(p.acc), 0, sizeof(double) * cl.total * Sc, st) != cudaSuccess) return LQGK_E_CUDA;
-    if (npad > n) {   // sums of padded samples are never written by k_trial_rev: zero them so k_cov_rev reads finite data
-      if (cudaMemsetAsync(F(p.sums) + (size_t)n * Tn * DM::SUMP, 0, sizeof(float) * (size_t)(npad - n) * Tn * DM::SUMP, st) != cudaSuccess)
-        return LQGK_E_CUDA;
-    }
-    if (warp_cov) {
-      size_t smem = BigW<DM>::smem_seq(), smemc = BigW<DM>::smem_con();
-      if ((rc = set_smem<DM>((const void*)kw_cov_seq_rev<DM>, smem))) return rc;
-      if ((rc = set_smem<DM>((const void*)kw_cov_contrib<DM, true>, smemc))) return rc;
-      {
-        ProfScope ps_(PK_COV_REV, st);
-        kw_cov_seq_rev<DM><<<wblk, 32 * BW_WARPS, smem, st>>>(npad, Tn, N, F(p.w), F(p.FU), F(p.JS), D(p.J0), F(p.sums), F(p.SGB), D(p.SGBI),
-                                                             F(p.SFW));
-        LQGK_LAUNCH_CHECK();
-      }
-      {
-        int chunks = std::max(1, std::min((Tn + 3) / 4, (sm_count() * 12 + npad - 1) / npad));
-        ProfScope ps_(PK_COV_CONTRIB, st);
-        kw_cov_contrib<DM, true><<<dim3(wblk, chunks), 32 * BW_WARPS, smemc, st>>>(D(p.cst), Sc, npad, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB),
-                                                                                  D(p.SGBI), F(p.SFW), F(p.sums), D(p.acc), D(p.Lbar), D(p.Kbar),
-                                                                                  D(p.KbarF));
-        LQGK_LAUNCH_CHECK();
-      }
-    } else {
-    {
-      size_t smem = smem_cov_seq_rev<DM>();
-      if ((rc = set_smem<DM>((const void*)k_cov_seq_rev<DM>, smem))) return rc;
-      ProfScope ps_(PK_COV_REV, st);
-      k_cov_seq_rev<DM><<<nblk, 32, smem, st>>>(Sc, Tn, N, F(p.w), F(p.FU), F(p.JS), D(p.J0), F(p.sums), F(p.SGB), D(p.SGBI), F(p.SFW), 0, Tn,
-                                                D(p.carC));
-      LQGK_LAUNCH_CHECK();
-    }
-    {
-      // (sample-group x time-range) warps: enough to occupy every SM a few times over
-      const int cwarps = g_contrib_warps > 0 ? g_contrib_warps : sm_count() * 30;
-      int chunks = std::max(1, std::min((Tn + 7) / 8, (cwarps + nblk - 1) / nblk));
-      dim3 grid(nblk, chunks);
-      if constexpr (contrib_merged<DM>()) {
-        size_t smem = smem_cov_contrib<DM, 2>();
-        if ((rc = set_smem<DM>((const void*)k_cov_contrib<DM, 2>, smem))) return rc;
-        ProfScope ps_(PK_COV_CONTRIB, st);
-        k_cov_contrib<DM, 2><<<grid, 32, smem, st>>>(D(p.cst), Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW), F(p.sums),
-                                                    D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), 0, Tn);
-        LQGK_LAUNCH_CHECK();
-      } else {
-        size_t smem0 = smem_cov_contrib<DM, 0>(), smem1 = smem_cov_contrib<DM, 1>();
-        if ((rc = set_smem<DM>((const void*)k_cov_contrib<DM, 0>, smem0))) return rc;
-        if ((rc = set_smem<DM>((const void*)k_cov_contrib<DM, 1>, smem1))) return rc;
-        a1 = (auxm & 2) ? x1 : st;
-        dep(st, a1);                               // cov_seq_rev done -> the two contraction passes run side by side
-        {
-          ProfScope ps_(PK_COV_CONTRIB, st);
-          k_cov_contrib<DM, 0><<<grid, 32, smem0, st>>>(D(p.cst), Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW),
-                                                       F(p.sums), D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), 0, Tn);
-          LQGK_LAUNCH_CHECK();
-        }
-        {
-          ProfScope ps_(PK_COV_CONTRIB, a1);
-          k_cov_contrib<DM, 1><<<grid, 32, smem1, a1>>>(D(p.cst), Sc, Tn, D(p.L), D(p.K), D(p.Cs), F(p.SGB), D(p.SGBI), F(p.SFW),
-                                                       F(p.sums), D(p.acc), D(p.Lbar), D(p.Kbar), D(p.KbarF), 0, Tn);
-          LQGK_LAUNCH_CHECK();
-        }
-      }
-    }
-    }   // !warp_cov
-    cudaEvent_t pass1_done = nullptr;
-    if (a1 != st) {
-      pass1_done = g_pool.next_event();
-      cudaEventRecord(pass1_done, a1);
-    }
-    if (!(auxm & 4)) {                             // no tail overlap: fold everything back onto st
-      dep(a1, st);
-      a1 = st;
-      pass1_done = nullptr;
-    } else {
-      a1 = x1;
-      a2 = x2;
-    }
-    dep(st, a2);                                   // pass 0 done -> Lbar complete -> Riccati adjoint on a2
-    {
-      size_t smem = smem_lqr_rev<DM>();
-      if ((rc = set_smem<DM>((const void*)k_lqr_rev<DM>, smem))) return rc;
-      ProfScope ps_(PK_LQR_REV, a2);
-      k_lqr_rev<DM><<<nblk, 32, smem, a2>>>(D(p.cst), Sc, Tn, c.eps, D(p.L), D(p.Sric), D(p.Lbar), D(p.acc));
-      LQGK_LAUNCH_CHECK();
-    }
-    if (pass1_done) cudaStreamWaitEvent(st, pass1_done, 0);   // Kbar parts complete -> Kalman adjoint on st
-    {
-      size_t smem = smem_kf_rev<DM>();
-      if ((rc = set_smem<DM>((const void*)k_kf_rev<DM>, smem))) return rc;
-      ProfScope ps_(PK_KF_REV, st);
-      k_kf_rev<DM><<<nblk, 32, smem, st>>>(D(p.cst), Sc, Tn, D(p.Pkf), D(p.Kbar), D(p.KbarF), D(p.acc), 0, Tn, D(p.carP));
-      LQGK_LAUNCH_CHECK();
-    }
-    dep(a1, st);
-    dep(a2, st);
-    {
-      UnpackArgs<T> ua{};
-      ua.act = *c.act; ua.dyn = *c.dyn; ua.sigma0 = pa.sigma0;
-      if (c.gact) ua.gact = *c.gact;
-      if (c.gdyn) ua.gdyn = *c.gdyn;
-      if (c.gsig0) ua.gsigma0 = *c.gsig0;
-      ua.x = DM::X; ua.b = DM::B; ua.u = DM::U; ua.y = DM::Y;
-      ProfScope ps_(PK_UNPACK, st);
-      k_unpack<T><<<(n + 63) / 64, 64, 0, st>>>(ua, (int)s0, n, D(p.acc), D(p.cst), Sc);
-      LQGK_LAUNCH_CHECK();
-    }
+    if ((rc = k.lqr_rev(x2))) return rc;         // after every contraction segment (Lbar complete), in order on x2
+    dep(x2, st);
+    dep(x3, st);
+    if ((rc = k.unpack(st))) return rc;
   }
   return LQGK_OK;
 }

@@ -43,7 +43,7 @@ def test_loglik_and_gradients_match_oracle(lib, dev, name, d, N):
 
 def test_large_system_c4(lib, dev):
     """BASELINE config c4 model: TemporalDelayModel(PointMassBoundedActor, delay=2): x=b=12, joint dim 24 -- the
-    large-system path (lqgk_big.cuh), 50 trials as in the config."""
+    large-system kernels (lqgk_bigw.cuh), 50 trials as in the config."""
     case = H.Case("pmdelay2", S=40, T=120, N=50, d=2, weights=True)
     H.check_gains(lib, dev, case, torch.float64, rtol=1e-9)
     H.check_fwd(lib, dev, case, torch.float32)
@@ -118,15 +118,16 @@ def test_config_c2_horizon(lib, dev):
 
 @pytest.mark.parametrize("name,d,N,T,reps", [("subjective", 2, 33, 205, 1), ("subjective", 2, 33, 205, 400), ("subjective2", 4, 40, 131, 1),
                                              ("bounded", 2, 301, 97, 200), ("delay2", 2, 20, 150, 1)])
-def test_pipelined_and_plain_launch_sequences_agree(lib, dev, name, d, N, T, reps):
-    """The pipelined launch sequence (time segments over internal streams; the default, so
-    every other test in this file runs it) and the plain one (what large sweeps use) are the same arithmetic: both match the
-    oracle, and each other to FP64-summation-order accuracy.  T is not a multiple of the checkpoint interval or the segment
-    count; reps > 1 tiles the samples beyond 512 to reach the thread-per-sample covariance kernels."""
+def test_one_segment_and_many_segments_agree(lib, dev, name, d, N, T, reps):
+    """The launch sequence cut into time segments over internal streams (the default, so every other test in this file runs
+    it) and its one-segment case on the caller's stream (pipeline off, or kernel overlap off) are the same arithmetic: all
+    match the oracle, and each other to FP64-summation-order accuracy.  T is not a multiple of the checkpoint interval or the
+    segment count; reps > 1 tiles the samples beyond 512 to reach the thread-per-sample covariance kernels."""
     case = H.Case(name, S=3, T=T, N=N, d=d, weights=True)
     outs = []
-    for max_samples, segments in ((0, 6), (1 << 20, 6), (1 << 20, 11), (1 << 20, 1000)):
+    for max_samples, segments, overlap in ((0, 6, 6), (1 << 20, 6, 6), (1 << 20, 11, 6), (1 << 20, 1000, 6), (1 << 20, 6, 0)):
         lib.set_pipeline(max_samples, min(segments, 64))
+        lib.set_kernel_overlap(overlap)
         try:
             if reps == 1:
                 H.check_vjp(lib, dev, case, torch.float32)
@@ -141,6 +142,7 @@ def test_pipelined_and_plain_launch_sequences_agree(lib, dev, name, d, N, T, rep
             outs.append([ll] + list(ga.values()) + list(gd.values()))
         finally:
             lib.set_pipeline(1 << 30, 6)
+            lib.set_kernel_overlap(6)
     for other in outs[1:]:
         for a, b in zip(outs[0], other):
             assert torch.allclose(a, b, rtol=1e-9, atol=1e-9 * float(a.abs().max()) + 1e-300)

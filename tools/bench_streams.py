@@ -1,5 +1,5 @@
 """Latency / strong-scaling regime: ms per log-likelihood+gradient through the public API as a function of the number of
-parameter samples and of the library's concurrent sample slices (lqgk_set_streams) and kernel-overlap mask.
+parameter samples and of the library's concurrent sample slices (lqgk_set_streams).
 python tools/bench_streams.py"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -33,14 +33,11 @@ def run(S, reps=5):
 
 
 streams = (1, 2, 4, 8, 16)
-print("| samples | " + " | ".join(f"{n} slices" for n in streams) + " | 1 slice, overlap 7 |\n|---:|" + "---:|" * (len(streams) + 1))
+print("| samples | " + " | ".join(f"{n} slices" for n in streams) + " |\n|---:|" + "---:|" * len(streams))
 for S in (512, 1024, 2048, 4096, 8192, 16384, 32768):
     row = []
     for n in streams:
         lib.set_streams(n)
         row.append(run(S))
     lib.set_streams(1)
-    lib.set_kernel_overlap(7)
-    row.append(run(S))
-    lib.set_kernel_overlap(6)
     print(f"| {S} | " + " | ".join(f"{v:.2f}" for v in row) + " |")
