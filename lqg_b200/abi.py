@@ -254,15 +254,12 @@ class Library:
         """LqgkSdnNoise from C_noise[S?, nc, x, u], D_noise[S?, nd, y, x] (None = none); tensors kept alive in `keep`."""
         nz = LqgkSdnNoise()
         for name, v, shp in (("C", C_noise, (dims.x, dims.u)), ("D", D_noise, (dims.y, dims.x))):
-            if v is None or v.numel() == 0:
-                setattr(nz, name, LqgkMat(None, 0, 0))
-                setattr(nz, "n" + name.lower(), 0)
+            if v is None or v.numel() == 0:   # (a fresh structure is zero: no matrix, no terms)
                 continue
             v = v.to(dt).contiguous()
             keep.append(v)
             assert tuple(v.shape[-2:]) == shp and v.dim() in (3, 4), (name, tuple(v.shape))
-            ss = v.stride(0) if v.dim() == 4 and v.shape[0] == dims.S and dims.S > 1 else 0
-            setattr(nz, name, LqgkMat(v.data_ptr(), ss, 0))
+            setattr(nz, name, _mat(v, dims.S, 1, trailing=3))
             setattr(nz, "n" + name.lower(), v.shape[-3])
         return nz
 
@@ -321,14 +318,11 @@ class Library:
         for k in base_nd:
             v = mats.get(k)
             if v is None or v.numel() == 0:
-                setattr(sp, k, LqgkMat(None, 0, 0))
                 continue
             assert v.dtype == torch.float64 and (v.is_cuda or not hasattr(self.lib, "lqgk_init")), k   # (host tensors: test harness only)
             v = v.contiguous()
             keep.append(v)
-            lead = v.dim() - base_nd[k]
-            ss = v.stride(0) if lead == 1 and v.shape[0] == S and S > 1 else 0
-            setattr(sp, k, LqgkMat(v.data_ptr(), ss, 0))
+            setattr(sp, k, _mat(v, S, 1, trailing=base_nd[k]))
         nc = 0 if mats.get("C") is None else mats["C"].shape[-3]
         nd = 0 if mats.get("D") is None else mats["D"].shape[-3]
         dims = LqgkSdnDims(S, T, b, u, y, nc, nd, sweeps)

@@ -7,7 +7,6 @@
 #include <cstdio>
 
 #include "../../include/lqgk.h"
-#include "lqgk_dims.h"
 #include "lqgk_run.cuh"
 
 using namespace lqgk;
@@ -27,45 +26,27 @@ thread_local int g_pipe_segments = 6;
 
 namespace {
 
-int validate(const Call& c) {
-  if (!c.dims || !c.act) return LQGK_E_INVALID;
-  const LqgkDims& d = *c.dims;
-  if (d.S <= 0 || d.T <= 0 || d.x <= 0 || d.b <= 0 || d.u <= 0 || d.y <= 0) return LQGK_E_INVALID;
-  if (!c.act->A.ptr || !c.act->B.ptr) return LQGK_E_INVALID;
-  if (c.mode != LQGK_MODE_GAINS) {
-    if (d.N <= 0 || d.d <= 0 || d.d > d.x) return LQGK_E_INVALID;
-    if (!c.dyn || !c.x_tm) return LQGK_E_INVALID;
-    if (c.mode == LQGK_MODE_MOMENTS ? (!c.mu_out && !c.Sig_out) : !c.ll_out) return LQGK_E_INVALID;
-    const LqgkMat* need[] = {&c.act->F, &c.act->V, &c.act->W, &c.act->Q, &c.act->R, &c.dyn->A, &c.dyn->B, &c.dyn->F, &c.dyn->V, &c.dyn->W};
-    for (auto m : need)
-      if (!m->ptr) return LQGK_E_INVALID;
-    if (((uintptr_t)c.x_tm % 16) != 0) return LQGK_E_INVALID;
-    // per-sample data sets: every sample's block must keep the alignment of the kernels' observation accesses (one d-float
-    // vector per trial: 16 bytes when d % 4 == 0, 8 when d % 2 == 0, else scalar loads)
-    const size_t xalign = d.d % 4 == 0 ? 16 : (d.d % 2 == 0 ? 8 : 4);
-    if (d.x_sample_stride < 0 || (d.x_sample_stride * sizeof(float)) % xalign != 0) return LQGK_E_INVALID;
-  }
-  return LQGK_OK;
+// (the workspace and stream come last, as in every entry point's parameters)
+template <class T>
+int dispatch(Call& c, void* ws, size_t ws_bytes, void* stream) {
+  g_launches = 0;
+  c.ws = ws; c.ws_bytes = ws_bytes; c.stream = (cudaStream_t)stream;
+  if (int rc = validate(c)) return rc;
+  return visit_tuple<Tuples::compiled>(call_key(*c.dims, c.mode), LQGK_E_UNSUPPORTED, [&](auto dm, auto) {
+    using R = Runner<decltype(dm)>;
+    return std::is_same<T, float>::value ? R::run_f32(c) : R::run_f64(c);
+  });
 }
 
-template <class T>
-int dispatch(const Call& c) {
-  g_launches = 0;
-  int rc = validate(c);
-  if (rc) return rc;
-  const LqgkDims& d = *c.dims;
-#define LQGK_CASE(X, B, U, Y, DD)                                                                       \
-  if (d.x == X && d.b == B && d.u == U && d.y == Y && (d.d == DD || c.mode == LQGK_MODE_GAINS))         \
-    return std::is_same<T, float>::value ? Runner<X, B, U, Y, DD>::run_f32(c) : Runner<X, B, U, Y, DD>::run_f64(c);
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return LQGK_E_UNSUPPORTED;
+size_t workspace_bytes(const LqgkDims& d, int mode, int32_t max_chunk) {
+  return visit_tuple<Tuples::compiled>(call_key(d, mode), (size_t)0,
+                                       [&](auto dm, auto) { return Runner<decltype(dm)>::plan_bytes(d, mode, max_chunk); });
 }
 
 template <class T>
 int pack_obs(int32_t N, int32_t T1, int32_t d, const T* x, float* x_tm, void* stream) {
   g_launches = 0;
-  if (N <= 0 || T1 <= 0 || d <= 0 || !x || !x_tm) return LQGK_E_INVALID;
+  if (int rc = check_pack_obs(N, T1, d, x, x_tm)) return rc;
   size_t total = (size_t)N * T1 * d;
   k_pack_obs<T><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(N, T1, d, x, x_tm);
   LQGK_LAUNCH_CHECK();
@@ -176,58 +157,34 @@ int simulate(const LqgkDims* d, const LqgkSpec* act, const LqgkSpec* dyn, const 
   if (!d || !act || !dyn || !L || !K || !x_out) return LQGK_E_INVALID;
   if (d->S <= 0 || d->N <= 0 || d->T <= 0 || d->x <= 0 || d->b <= 0 || d->u <= 0 || d->y <= 0) return LQGK_E_INVALID;
   if (d->x > SIM_MAX || d->b > SIM_MAX || d->u > SIM_MAX || d->y > SIM_MAX) return LQGK_E_UNSUPPORTED;
-  const LqgkMat* need[] = {&act->A, &act->B, &act->F, &dyn->A, &dyn->B, &dyn->F, &dyn->V, &dyn->W};
-  for (auto m : need)
-    if (!m->ptr) return LQGK_E_INVALID;
+  if (need_closed_loop(*act, *dyn, false) || check_noise(nz)) return LQGK_E_INVALID;
   SimArgs<T> a{*act, *dyn, L, l, K, x0, xhat0, x_out, xhat_out, y_out, u_out, d->S, d->N, d->T, d->x, d->b, d->u, d->y, seed};
   a.Cn = LqgkMat{nullptr, 0, 0}; a.Dn = LqgkMat{nullptr, 0, 0}; a.nc = 0; a.nd = 0;
-  if (nz) {
-    if (nz->nc < 0 || nz->nd < 0 || nz->nc > SDN_MAX_TERMS || nz->nd > SDN_MAX_TERMS) return LQGK_E_INVALID;
-    if ((nz->nc > 0 && !nz->C.ptr) || (nz->nd > 0 && !nz->D.ptr)) return LQGK_E_INVALID;
-    a.Cn = nz->C; a.Dn = nz->D; a.nc = nz->nc; a.nd = nz->nd;
-  }
+  if (nz) { a.Cn = nz->C; a.Dn = nz->D; a.nc = nz->nc; a.nd = nz->nd; }
   const size_t total = (size_t)d->S * d->N;
   k_simulate<T><<<(unsigned)((total + 63) / 64), 64, 0, (cudaStream_t)stream>>>(a);
   LQGK_LAUNCH_CHECK();
   return LQGK_OK;
 }
-}  // namespace
 
-namespace {
 int sdn_loglik(const LqgkDims* d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkSdnNoise* nz, const void* L, const void* K,
                const float* x_tm, void* ll_out, bool f64, void* stream) {
   g_launches = 0;
-  if (!d || !act || !dyn || !L || !K || !x_tm || !ll_out) return LQGK_E_INVALID;
-  if (d->S <= 0 || d->N <= 0 || d->T <= 0 || d->d <= 0 || d->d > d->x || d->x_sample_stride < 0) return LQGK_E_INVALID;
-  const LqgkMat* need[] = {&act->A, &act->B, &act->F, &dyn->A, &dyn->B, &dyn->F, &dyn->V, &dyn->W};
-  for (auto m : need) {
-    if (!m->ptr) return LQGK_E_INVALID;
-    if (m->time_stride != 0) return LQGK_E_UNSUPPORTED;
-  }
-  SdnLikArgs a{};
-  a.act = *act; a.dyn = *dyn; a.L = L; a.K = K; a.x_tm = x_tm; a.x_sample_stride = d->x_sample_stride; a.ll_out = ll_out;
-  a.S = d->S; a.N = d->N; a.T = d->T;
-  if (nz) {
-    if (nz->nc < 0 || nz->nd < 0 || nz->nc > SDN_MAX_TERMS || nz->nd > SDN_MAX_TERMS) return LQGK_E_INVALID;
-    if ((nz->nc > 0 && !nz->C.ptr) || (nz->nd > 0 && !nz->D.ptr)) return LQGK_E_INVALID;
-    a.C = nz->C; a.D = nz->D; a.nc = nz->nc; a.nd = nz->nd;
-  }
-#define LQGK_CASE(X, B, U, Y, DD) \
-  if (d->x == X && d->b == B && d->u == U && d->y == Y && d->d == DD) return Runner<X, B, U, Y, DD>::run_sdn_loglik(a, f64, (cudaStream_t)stream);
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  // tuples compiled for this all-FP64 path only (lqgk_dims.h)
-#define LQGK_CASE(X, B, U, Y, DD)                                                                        \
-  if (d->x == X && d->b == B && d->u == U && d->y == Y && d->d == DD) {                                  \
-    const unsigned blocks = (unsigned)(((size_t)a.S * a.N + 63) / 64);                                   \
-    if (f64) k_sdn_loglik<Dims<X, B, U, Y, DD>, double><<<blocks, 64, 0, (cudaStream_t)stream>>>(a);      \
-    else k_sdn_loglik<Dims<X, B, U, Y, DD>, float><<<blocks, 64, 0, (cudaStream_t)stream>>>(a);           \
-    LQGK_LAUNCH_CHECK();                                                                                 \
-    return LQGK_OK;                                                                                      \
-  }
-  LQGK_FOR_EACH_FP64_ONLY_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return LQGK_E_UNSUPPORTED;
+  SdnLikArgs a;
+  if (int rc = sdn_lik_args(d, act, dyn, nz, L, K, x_tm, ll_out, a)) return rc;
+  // the tuples of the main path launch from their own objects (lqgk_inst.cu), the FP64-only ones from this one
+  return visit_tuple<Tuples::small_and_fp64_only>(full_key(*d), LQGK_E_UNSUPPORTED, [&](auto dm, auto fp64_only) {
+    using DM = decltype(dm);
+    if constexpr (decltype(fp64_only)::value) return launch_sdn_loglik<DM>(a, f64, (cudaStream_t)stream);
+    else return Runner<DM>::run_sdn_loglik(a, f64, (cudaStream_t)stream);
+  });
+}
+int sdn_gains(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, void* stream, int filter_form) {
+  g_launches = 0;
+  SdnArgs a;
+  if (int rc = sdn_gains_args(d, sp, L_out, K_out, cost_out, filter_form, a)) return rc;
+  return visit_tuple<Tuples::small>(TupleKey{ANY, d->b, d->u, d->y, ANY}, LQGK_E_UNSUPPORTED,
+                                    [&](auto dm, auto) { return Runner<decltype(dm)>::run_sdn(a, (cudaStream_t)stream); });
 }
 }  // namespace
 
@@ -250,43 +207,11 @@ __global__ void k_peak_fma(int iters, T* sink) {
 }
 extern "C" {
 
-static int sdn_gains_impl(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, void* stream, int filter_form) {
-  g_launches = 0;
-  if (!d || !sp || !L_out || !K_out) return LQGK_E_INVALID;
-  if (d->S <= 0 || d->T <= 0 || d->b <= 0 || d->u <= 0 || d->y <= 0 || d->nc < 0 || d->nd < 0 || d->sweeps < 0) return LQGK_E_INVALID;
-  const LqgkMat* need[] = {&sp->A, &sp->B, &sp->H, &sp->Q, &sp->R, &sp->Om_xi, &sp->Om_omega, &sp->Sigma1};
-  for (auto m : need)
-    if (!m->ptr) return LQGK_E_INVALID;
-  if ((d->nc > 0 && !sp->C.ptr) || (d->nd > 0 && !sp->D.ptr)) return LQGK_E_INVALID;
-  SdnArgs a{};
-  auto P = [](const LqgkMat& m) { return (const double*)m.ptr; };
-  a.A = P(sp->A); a.sA = sp->A.sample_stride;
-  a.B = P(sp->B); a.sB = sp->B.sample_stride;
-  a.H = P(sp->H); a.sH = sp->H.sample_stride;
-  a.C = P(sp->C); a.sC = sp->C.sample_stride;
-  a.D = P(sp->D); a.sD = sp->D.sample_stride;
-  a.Q = P(sp->Q); a.sQ = sp->Q.sample_stride;
-  a.R = P(sp->R); a.sR = sp->R.sample_stride;
-  a.Qf = sp->Qf.ptr ? P(sp->Qf) : P(sp->Q); a.sQf = sp->Qf.ptr ? sp->Qf.sample_stride : sp->Q.sample_stride;
-  a.Omxi = P(sp->Om_xi); a.sOmxi = sp->Om_xi.sample_stride;
-  a.Omom = P(sp->Om_omega); a.sOmom = sp->Om_omega.sample_stride;
-  a.Sig1 = P(sp->Sigma1); a.sSig1 = sp->Sigma1.sample_stride;
-  if (!sp->xhat1.ptr) return LQGK_E_INVALID;
-  a.xh1 = P(sp->xhat1); a.sxh1 = sp->xhat1.sample_stride;
-  a.S = d->S; a.T = d->T; a.nc = d->nc; a.nd = d->nd; a.sweeps = d->sweeps;
-  a.L = L_out; a.K = K_out; a.cost = cost_out; a.filter_form = filter_form;
-#define LQGK_CASE(X, B, U, Y, DD) \
-  if (X + B <= 12 && d->b == B && d->u == U && d->y == Y) return Runner<X, B, U, Y, DD>::run_sdn(a, (cudaStream_t)stream);
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return LQGK_E_UNSUPPORTED;
-}
-
 int lqgk_sdn_gains_f64(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, void* stream) {
-  return sdn_gains_impl(d, sp, L_out, K_out, cost_out, stream, 0);
+  return sdn_gains(d, sp, L_out, K_out, cost_out, stream, 0);
 }
 int lqgk_sdn_gains_filter_f64(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, void* stream) {
-  return sdn_gains_impl(d, sp, L_out, K_out, cost_out, stream, 1);
+  return sdn_gains(d, sp, L_out, K_out, cost_out, stream, 1);
 }
 
 int lqgk_sdn_loglik_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkSdnNoise* noise, const float* L,
@@ -300,62 +225,70 @@ int lqgk_sdn_loglik_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkS
 
 int lqgk_lqr_backward_f32(const LqgkDims* dims, const LqgkSpec* actor, double eps, float* L_out, float* l_out, float* H_out,
                           void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, L_out, l_out, H_out, nullptr, eps, LQGK_MODE_GAINS, ws, ws_bytes, (cudaStream_t)stream};
-  if (!L_out) return LQGK_E_INVALID;
-  return dispatch<float>(c);
+  Call c;
+  c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.eps = eps; c.L_out = L_out; c.l_out = l_out; c.H_out = H_out;
+  return dispatch<float>(c, ws, ws_bytes, stream);
 }
 int lqgk_lqr_backward_f64(const LqgkDims* dims, const LqgkSpec* actor, double eps, double* L_out, double* l_out, double* H_out,
                           void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, L_out, l_out, H_out, nullptr, eps, LQGK_MODE_GAINS, ws, ws_bytes, (cudaStream_t)stream};
-  if (!L_out) return LQGK_E_INVALID;
-  return dispatch<double>(c);
+  Call c;
+  c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.eps = eps; c.L_out = L_out; c.l_out = l_out; c.H_out = H_out;
+  return dispatch<double>(c, ws, ws_bytes, stream);
 }
 int lqgk_kf_forward_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, float* K_out, void* ws,
                         size_t ws_bytes, void* stream) {
-  Call c{dims, actor, nullptr, sigma0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, K_out, 1e-8, LQGK_MODE_GAINS, ws, ws_bytes, (cudaStream_t)stream};
-  if (!K_out) return LQGK_E_INVALID;
-  return dispatch<float>(c);
+  Call c;
+  c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.sigma0 = sigma0; c.K_out = K_out;
+  return dispatch<float>(c, ws, ws_bytes, stream);
 }
 int lqgk_kf_forward_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double* K_out, void* ws,
                         size_t ws_bytes, void* stream) {
-  Call c{dims, actor, nullptr, sigma0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, K_out, 1e-8, LQGK_MODE_GAINS, ws, ws_bytes, (cudaStream_t)stream};
-  if (!K_out) return LQGK_E_INVALID;
-  return dispatch<double>(c);
+  Call c;
+  c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.sigma0 = sigma0; c.K_out = K_out;
+  return dispatch<double>(c, ws, ws_bytes, stream);
 }
 int lqgk_loglik_fwd_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, float* ll_out, void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, dynamics, sigma0, x_tm, nullptr, ll_out, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_FWD, ws, ws_bytes, (cudaStream_t)stream};
-  return dispatch<float>(c);
+  Call c;
+  c.mode = LQGK_MODE_FWD; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_out = ll_out;
+  return dispatch<float>(c, ws, ws_bytes, stream);
 }
 int lqgk_loglik_fwd_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, double* ll_out, void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, dynamics, sigma0, x_tm, nullptr, ll_out, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_FWD, ws, ws_bytes, (cudaStream_t)stream};
-  return dispatch<double>(c);
+  Call c;
+  c.mode = LQGK_MODE_FWD; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_out = ll_out;
+  return dispatch<double>(c, ws, ws_bytes, stream);
 }
 int lqgk_loglik_vjp_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, const float* ll_bar, float* ll_out, const LqgkSpecGrad* ga, const LqgkSpecGrad* gd,
                         const LqgkMatGrad* gs, void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, dynamics, sigma0, x_tm, ll_bar, ll_out, ga, gd, gs, nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_VJP, ws, ws_bytes, (cudaStream_t)stream};
-  return dispatch<float>(c);
+  Call c;
+  c.mode = LQGK_MODE_VJP; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_bar = ll_bar;
+  c.ll_out = ll_out; c.gact = ga; c.gdyn = gd; c.gsig0 = gs;
+  return dispatch<float>(c, ws, ws_bytes, stream);
 }
 int lqgk_loglik_vjp_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, const double* ll_bar, double* ll_out, const LqgkSpecGrad* ga, const LqgkSpecGrad* gd,
                         const LqgkMatGrad* gs, void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, dynamics, sigma0, x_tm, ll_bar, ll_out, ga, gd, gs, nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_VJP, ws, ws_bytes, (cudaStream_t)stream};
-  return dispatch<double>(c);
+  Call c;
+  c.mode = LQGK_MODE_VJP; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_bar = ll_bar;
+  c.ll_out = ll_out; c.gact = ga; c.gdyn = gd; c.gsig0 = gs;
+  return dispatch<double>(c, ws, ws_bytes, stream);
 }
 
 int lqgk_moments_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0, const float* x_tm,
                      float* mu_out, float* Sigma_out, void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, dynamics, sigma0, x_tm, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_MOMENTS, ws, ws_bytes, (cudaStream_t)stream};
-  c.mu_out = mu_out; c.Sig_out = Sigma_out;
-  return dispatch<float>(c);
+  Call c;
+  c.mode = LQGK_MODE_MOMENTS; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.mu_out = mu_out;
+  c.Sig_out = Sigma_out;
+  return dispatch<float>(c, ws, ws_bytes, stream);
 }
 int lqgk_moments_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0, const float* x_tm,
                      double* mu_out, double* Sigma_out, void* ws, size_t ws_bytes, void* stream) {
-  Call c{dims, actor, dynamics, sigma0, x_tm, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_MOMENTS, ws, ws_bytes, (cudaStream_t)stream};
-  c.mu_out = mu_out; c.Sig_out = Sigma_out;
-  return dispatch<double>(c);
+  Call c;
+  c.mode = LQGK_MODE_MOMENTS; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.mu_out = mu_out;
+  c.Sig_out = Sigma_out;
+  return dispatch<double>(c, ws, ws_bytes, stream);
 }
 int lqgk_simulate_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const float* L, const float* l, const float* K,
                       const float* x0, const float* xhat0, uint64_t seed, float* x_out, float* xhat_out, float* y_out, float* u_out,
@@ -387,24 +320,11 @@ int lqgk_pack_obs_f64(int32_t N, int32_t T1, int32_t d, const double* x, float* 
 }
 
 size_t lqgk_workspace_bytes(const LqgkDims* dims, int mode, int32_t max_chunk) {
-  if (!dims) return 0;
-  const LqgkDims& d = *dims;
-#define LQGK_CASE(X, B, U, Y, DD)                                                              \
-  if (d.x == X && d.b == B && d.u == U && d.y == Y && (d.d == DD || mode == LQGK_MODE_GAINS)) \
-    return Runner<X, B, U, Y, DD>::plan_bytes(d, mode, max_chunk);
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return 0;
+  return dims ? workspace_bytes(*dims, mode, max_chunk) : 0;
 }
 
 int lqgk_dims_supported(const LqgkDims* dims) {
-  if (!dims) return 0;
-  const LqgkDims& d = *dims;
-#define LQGK_CASE(X, B, U, Y, DD) \
-  if (d.x == X && d.b == B && d.u == U && d.y == Y && d.d == DD) return 1;
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return 0;
+  return dims && visit_tuple<Tuples::compiled>(full_key(*dims), 0, [](auto, auto) { return 1; });
 }
 
 const char* lqgk_strerror(int code) {

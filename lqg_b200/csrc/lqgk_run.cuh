@@ -9,6 +9,7 @@
 #include "../../include/lqgk.h"
 #include "lqgk_kernels.cuh"
 #include "lqgk_bigw.cuh"
+#include "lqgk_entry.h"
 #include "lqgk_sdn.cuh"
 
 namespace lqgk {
@@ -143,14 +144,6 @@ extern thread_local int g_warp_cov_max_samples;   // calls with at most this man
 extern thread_local int g_pipe_max_samples, g_pipe_segments;
 inline size_t up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-inline bool spec_time_varying(const LqgkSpec& s, bool actor) {
-  const LqgkMat* m[] = {&s.A, &s.B, &s.F, &s.V, &s.W, &s.Q, &s.R, &s.q, &s.r, &s.P};
-  int n = actor ? 10 : 5;
-  for (int i = 0; i < n; ++i)
-    if (m[i]->ptr && m[i]->time_stride != 0) return true;
-  return false;
-}
-
 // Large systems (joint dim > 12) take the warp-per-sample kernels of lqgk_bigw.cuh (see the kernel launchers below).
 template <class DM>
 constexpr bool is_big() { return DM::N > 12; }
@@ -262,26 +255,6 @@ int launch_trial_rev(cudaStream_t st, const float* rec, const float* xc, size_t 
   LQGK_LAUNCH_CHECK();
   return LQGK_OK;
 }
-
-struct Call {
-  const LqgkDims* dims;
-  const LqgkSpec* act;
-  const LqgkSpec* dyn;
-  const LqgkMat* sigma0;
-  const float* x_tm;
-  const void* ll_bar;
-  void* ll_out;
-  const LqgkSpecGrad* gact;
-  const LqgkSpecGrad* gdyn;
-  const LqgkMatGrad* gsig0;
-  void *L_out, *l_out, *H_out, *K_out;
-  double eps;
-  int mode;
-  void* ws;
-  size_t ws_bytes;
-  cudaStream_t stream;
-  void *mu_out = nullptr, *Sig_out = nullptr;   // moments entry point
-};
 
 // ------------------------------------------------------------------------------------------------------- kernel launchers
 // One launcher per stage of the likelihood path.  A launcher takes its stream and, for a sweep over time, the range of one
@@ -600,9 +573,7 @@ int run(const Call& c) {
   const LqgkDims& d = *c.dims;
   const bool has_dyn = c.dyn != nullptr;
   const bool tv = spec_time_varying(*c.act, true) || (has_dyn && spec_time_varying(*c.dyn, false));
-  if (tv && c.mode == LQGK_MODE_VJP) return LQGK_E_UNSUPPORTED;
-  // large systems: no time-varying specs, and the predictive moments stay on the host-side slow path
-  if (is_big<DM>() && (tv || c.mode == LQGK_MODE_MOMENTS)) return LQGK_E_UNSUPPORTED;
+  if (!kernels_cover(c, tv, is_big<DM>())) return LQGK_E_UNSUPPORTED;
   if (!c.ws || ((uintptr_t)c.ws % ALIGN) != 0) return LQGK_E_INVALID;
   // slices: ns concurrent streams, each with its own workspace part and chunk size Sc
   int ns = c.mode == LQGK_MODE_GAINS ? 1 : std::max(1, std::min(g_streams, (int)((d.S + 31) / 32)));
@@ -755,9 +726,18 @@ int run(const Call& c) {
   return LQGK_OK;
 }
 
+// The per-trial likelihood under signal-dependent noise, all FP64 (small and FP64-only tuples): one thread per (sample, trial).
+template <class DM>
+int launch_sdn_loglik(const SdnLikArgs& a, bool f64, cudaStream_t st) {
+  const unsigned blocks = (unsigned)(((size_t)a.S * a.N + 63) / 64);
+  if (f64) k_sdn_loglik<DM, double><<<blocks, 64, 0, st>>>(a);
+  else k_sdn_loglik<DM, float><<<blocks, 64, 0, st>>>(a);
+  LQGK_LAUNCH_CHECK();
+  return LQGK_OK;
+}
 
-// One specialisation per compiled dimension tuple (defined in lqgk_inst.cu).
-template <int X, int B, int U, int Y, int D>
+// One specialisation per line of LQGK_FOR_EACH_DIMS (defined in lqgk_inst.cu; run_sdn* for joint dims <= 12 only).
+template <class DM>
 struct Runner {
   static int run_f32(const Call& c);
   static int run_f64(const Call& c);

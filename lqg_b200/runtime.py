@@ -92,6 +92,26 @@ def spec_mats(spec: LQGSpec, keys) -> Dict[str, torch.Tensor]:
     return {k: _row_major(_as4(getattr(spec, k))) for k in keys}
 
 
+def _untimed(M: torch.Tensor, dt) -> torch.Tensor:
+    """(S|1, r, c) row-major in dtype dt from a matrix without time axis (Qf, Sigma0) shaped (r, c) or (S, r, c)."""
+    return _row_major(M if M.dim() == 3 else M.unsqueeze(0)).to(dt)
+
+
+def _per_sample(t: Optional[torch.Tensor], nd: int, S: int, dt) -> Optional[torch.Tensor]:
+    """Gains with an optional leading sample axis (nd dims without it) -> (S, ...) contiguous."""
+    if t is None:
+        return None
+    t = t if t.dim() == nd + 1 else t.unsqueeze(0)
+    return t.expand(S, *t.shape[1:]).to(dt).contiguous()
+
+
+def _unbatch(actor: LQGSpec, dynamics: LQGSpec, out):
+    """Drops the sample axis of a call's output(s) (a tensor, or a tuple of tensors and Nones) for an un-batched model."""
+    if not (actor.A.dim() == 3 and dynamics.A.dim() == 3):
+        return out
+    return tuple(o[0] if o is not None else None for o in out) if isinstance(out, tuple) else out[0]
+
+
 def is_time_invariant(M4: torch.Tensor) -> bool:
     return M4.shape[1] == 1 or M4.stride(1) == 0
 
@@ -123,16 +143,28 @@ def _stream(device):
     return torch.cuda.current_stream(device).cuda_stream
 
 
-def lqr_backward(spec: LQGSpec, eps: float = 1e-8):
-    """CUDA backward Riccati sweep.  Returns L, l, H shaped like the reference ((T,u,b) or (S,T,u,b))."""
-    _require_cuda(spec.A, "spec")
-    lib = abi.load_library()
+def _gains_dims(spec: LQGSpec) -> abi.LqgkDims:
+    """Dimensions of a gains-only call.  The sweeps read the actor's (b, u, y) only: x and d are those of the first compiled
+    tuple with that (b, u, y), or (b, 1) when there is none (check_supported then refuses the call)."""
     S, T = spec_batch(spec)
     b, u, y = spec.A.shape[-1], spec.B.shape[-1], spec.F.shape[-2]
-    dims = abi.LqgkDims(S, 1, T, next((t[0] for t in SUPPORTED_DIMS if t[1:4] == (b, u, y)), b), b, u, y, 1)
-    dims.d = next((t[4] for t in SUPPORTED_DIMS if t[:4] == (dims.x, b, u, y)), 1)
+    x, d = next(((t[0], t[4]) for t in SUPPORTED_DIMS if t[1:4] == (b, u, y)), (b, 1))
+    return abi.LqgkDims(S, 1, T, x, b, u, y, d)
+
+
+def _gains_call(spec: LQGSpec):
+    """What lqr_backward and kf_forward share: the library, the dimensions, the actor's matrices and the workspace."""
+    _require_cuda(spec.A, "spec")
+    lib = abi.load_library()
+    dims = _gains_dims(spec)
     check_supported(dims, gains_only=True)
-    mats = spec_mats(spec, ACT_KEYS)
+    ws = workspace(spec.A.device, lib.workspace_bytes(dims, abi.MODE_GAINS, 0))
+    return lib, dims, spec_mats(spec, ACT_KEYS), ws
+
+
+def lqr_backward(spec: LQGSpec, eps: float = 1e-8):
+    """CUDA backward Riccati sweep.  Returns L, l, H shaped like the reference ((T,u,b) or (S,T,u,b))."""
+    lib, dims, mats, ws = _gains_call(spec)
     # affine terms are always handed to the kernel (zeros in every reference model): no host-side "is it zero?" sync
     for k, tr in (("q", 1), ("r", 1), ("P", 2)):
         v = getattr(spec, k)
@@ -142,10 +174,8 @@ def lqr_backward(spec: LQGSpec, eps: float = 1e-8):
     if spec.qf is not None:
         mats["qf"] = (spec.qf if spec.qf.dim() == 2 else spec.qf.unsqueeze(0)).contiguous()
     if spec.Qf is not None:
-        mats["Qf"] = _row_major(spec.Qf if spec.Qf.dim() == 3 else spec.Qf.unsqueeze(0))
-    dev = spec.A.device
-    ws = workspace(dev, lib.workspace_bytes(dims, abi.MODE_GAINS, 0))
-    L, l, H = lib.lqr_backward(dims, mats, eps=eps, ws=ws, stream=_stream(dev))
+        mats["Qf"] = _untimed(spec.Qf, spec.A.dtype)
+    L, l, H = lib.lqr_backward(dims, mats, eps=eps, ws=ws, stream=_stream(spec.A.device))
     if spec.A.dim() == 3:
         L, l, H = L[0], l[0], H[0]
     return L, l, H
@@ -153,20 +183,9 @@ def lqr_backward(spec: LQGSpec, eps: float = 1e-8):
 
 def kf_forward(spec: LQGSpec, Sigma0: Optional[torch.Tensor]):
     """CUDA forward Kalman-gain sweep.  Returns K shaped (T,b,y) or (S,T,b,y)."""
-    _require_cuda(spec.A, "spec")
-    lib = abi.load_library()
-    S, T = spec_batch(spec)
-    b, u, y = spec.A.shape[-1], spec.B.shape[-1], spec.F.shape[-2]
-    dims = abi.LqgkDims(S, 1, T, next((t[0] for t in SUPPORTED_DIMS if t[1:4] == (b, u, y)), b), b, u, y, 1)
-    dims.d = next((t[4] for t in SUPPORTED_DIMS if t[:4] == (dims.x, b, u, y)), 1)
-    check_supported(dims, gains_only=True)
-    mats = spec_mats(spec, ACT_KEYS)
-    dev = spec.A.device
-    s0 = None
-    if Sigma0 is not None:
-        s0 = _row_major(Sigma0 if Sigma0.dim() == 3 else Sigma0.unsqueeze(0)).to(spec.A.dtype)
-    ws = workspace(dev, lib.workspace_bytes(dims, abi.MODE_GAINS, 0))
-    K = lib.kf_forward(dims, mats, sigma0=s0, ws=ws, stream=_stream(dev))
+    lib, dims, mats, ws = _gains_call(spec)
+    s0 = None if Sigma0 is None else _untimed(Sigma0, spec.A.dtype)
+    K = lib.kf_forward(dims, mats, sigma0=s0, ws=ws, stream=_stream(spec.A.device))
     return K[0] if spec.A.dim() == 3 else K
 
 
@@ -267,6 +286,31 @@ def _check_no_cross_cost(actor: LQGSpec):
                                   "use lqr.backward / conditional_moments (slow path) for specs with P != 0")
 
 
+def _observed_call(lib, dims: abi.LqgkDims, actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, Sigma0, call, x_tm=None):
+    """Checks x[(S,) n, T+1, d] against the spec, packs it (unless x_tm is given), hands the base matrices (with a Qf of the
+    spec's own) and Sigma0 to ``call(x_tm, act, dyn, sigma0)`` and drops the sample axis of its output for an un-batched model."""
+    per_sample = x.dim() == 4
+    if per_sample and x.shape[0] != dims.S:
+        raise ValueError(f"per-sample observations need a leading axis of {dims.S} samples, got {x.shape[0]}")
+    if dims.T != x.shape[-2] - 1:
+        raise ValueError(f"need T+1 = {dims.T + 1} observations per trial, got {x.shape[-2]} (SURVEY H7: spec.T == x.shape[-2] - 1)")
+    if x_tm is None:
+        if per_sample:   # [S, n, T+1, d] -> [S, T+1, n, d] float32
+            x_tm = x.detach().permute(0, 2, 1, 3).to(torch.float32).contiguous()
+        else:
+            x_tm = lib.pack_obs(x.detach(), stream=_stream(x.device))
+    dt = actor.A.dtype
+
+    def base(M):   # (S|1, r, c) base matrix of a time-invariant array (stride-0 time axis), else the (S|1, T, r, c) array
+        M4 = _as4(M)
+        return _row_major(M4[:, 0] if is_time_invariant(M4) else M4).to(dt)
+    act, dyn = {k: base(getattr(actor, k)) for k in ACT_KEYS}, {k: base(getattr(dynamics, k)) for k in DYN_KEYS}
+    if not _qf_is_default(actor):   # a terminal cost of its own (lqg/control/lqr.py:37 starts the sweep from spec.Qf)
+        act["Qf"] = _untimed(actor.Qf, dt)
+    s0 = None if Sigma0 is None else _untimed(Sigma0, dt)
+    return _unbatch(actor, dynamics, call(x_tm, act, dyn, s0))
+
+
 def log_likelihood(actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, Sigma0: Optional[torch.Tensor] = None,
                    x_tm: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Per-trial log-likelihood (reference ``System.log_likelihood``, lqg/system.py:246-248).
@@ -276,43 +320,14 @@ def log_likelihood(actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, Sigma0: O
     _require_cuda(actor.A, "actor spec")
     _require_cuda(x, "observations")
     lib = abi.load_library()
-    per_sample = x.dim() == 4
-    n, T1, d = x.shape[-3:]
-    dims = dims_of(actor, dynamics, n, d)
-    if per_sample and x.shape[0] != dims.S:
-        raise ValueError(f"per-sample observations need a leading axis of {dims.S} samples, got {x.shape[0]}")
-    if dims.T != T1 - 1:
-        raise ValueError(f"need T+1 = {dims.T + 1} observations per trial, got {T1} (SURVEY H7: spec.T == x.shape[-2] - 1)")
+    dims = dims_of(actor, dynamics, x.shape[-3], x.shape[-1])
     check_supported(dims)
     _check_no_cross_cost(actor)
-    if x_tm is None:
-        if per_sample:   # [S, n, T+1, d] -> [S, T+1, n, d] float32
-            x_tm = x.detach().permute(0, 2, 1, 3).to(torch.float32).contiguous()
-        else:
-            x_tm = lib.pack_obs(x.detach(), stream=_stream(x.device))
-    dt = actor.A.dtype
-    def base(M):
-        """(S|1, r, c) base matrix of a time-invariant array (stride-0 time axis), else the (S|1, T, r, c) array."""
-        M4 = _as4(M)
-        return _row_major(M4[:, 0] if is_time_invariant(M4) else M4).to(dt)
 
-    mats = [base(getattr(actor, k)) for k in ACT_KEYS] + [base(getattr(dynamics, k)) for k in DYN_KEYS]
-    has_qf = not _qf_is_default(actor)
-    if has_qf:   # a terminal cost of its own (lqg/control/lqr.py:37 starts the sweep from spec.Qf)
-        Qf = actor.Qf
-        mats.append(_row_major(Qf if Qf.dim() == 3 else Qf.unsqueeze(0)).to(dt))
-    has_s0 = Sigma0 is not None
-    if has_s0:
-        mats.append(_row_major(Sigma0 if Sigma0.dim() == 3 else Sigma0.unsqueeze(0)).to(dt))
-    ll = _LogLikFn.apply(x_tm, dims, has_qf, has_s0, len(ACT_KEYS), *mats)
-    return ll[0] if (actor.A.dim() == 3 and dynamics.A.dim() == 3) else ll
-
-
-def _base_mats(actor: LQGSpec, dynamics: LQGSpec, dt):
-    def base(M):
-        M4 = _as4(M)
-        return _row_major(M4[:, 0] if is_time_invariant(M4) else M4).to(dt)
-    return {k: base(getattr(actor, k)) for k in ACT_KEYS}, {k: base(getattr(dynamics, k)) for k in DYN_KEYS}
+    def call(x_tm, act, dyn, s0):
+        mats = [act[k] for k in ACT_KEYS] + [dyn[k] for k in DYN_KEYS] + [m for m in (act.get("Qf"), s0) if m is not None]
+        return _LogLikFn.apply(x_tm, dims, "Qf" in act, s0 is not None, len(ACT_KEYS), *mats)
+    return _observed_call(lib, dims, actor, dynamics, x, Sigma0, call, x_tm=x_tm)
 
 
 def moments(actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, Sigma0: Optional[torch.Tensor] = None, want_mu=True, want_sigma=True):
@@ -326,19 +341,12 @@ def moments(actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, Sigma0: Optional
     if (dims.x, dims.b, dims.u, dims.y, dims.d) not in SUPPORTED_DIMS or dims.x + dims.b > 12 or dims.T != T1 - 1:
         return None
     _check_no_cross_cost(actor)
-    dt = actor.A.dtype
-    act, dyn = _base_mats(actor, dynamics, dt)
-    if not _qf_is_default(actor):
-        Qf = actor.Qf
-        act["Qf"] = _row_major(Qf if Qf.dim() == 3 else Qf.unsqueeze(0)).to(dt)
-    x_tm = lib.pack_obs(x.detach(), stream=_stream(x.device)) if x.dim() == 3 else x.detach().permute(0, 2, 1, 3).to(torch.float32).contiguous()
-    s0 = None if Sigma0 is None else _row_major(Sigma0 if Sigma0.dim() == 3 else Sigma0.unsqueeze(0)).to(dt)
     dev = actor.A.device
-    ws = workspace(dev, lib.workspace_bytes(dims, abi.MODE_MOMENTS, 0))
-    mu, Sig = lib.moments(dims, act, dyn, x_tm, sigma0=s0, want_mu=want_mu, want_sigma=want_sigma, ws=ws, stream=_stream(dev))
-    if actor.A.dim() == 3 and dynamics.A.dim() == 3:
-        mu, Sig = (mu[0] if mu is not None else None), (Sig[0] if Sig is not None else None)
-    return mu, Sig
+
+    def call(x_tm, act, dyn, s0):
+        ws = workspace(dev, lib.workspace_bytes(dims, abi.MODE_MOMENTS, 0))
+        return lib.moments(dims, act, dyn, x_tm, sigma0=s0, want_mu=want_mu, want_sigma=want_sigma, ws=ws, stream=_stream(dev))
+    return _observed_call(lib, dims, actor, dynamics, x, Sigma0, call)
 
 
 def simulate(actor: LQGSpec, dynamics: LQGSpec, L, l, K, n: int, seed: int, x0=None, xhat0=None, return_all=False, C=None, D=None):
@@ -355,18 +363,11 @@ def simulate(actor: LQGSpec, dynamics: LQGSpec, L, l, K, n: int, seed: int, x0=N
     act = {k: _row_major(_as4(getattr(actor, k))).to(dt) for k in ("A", "B", "F")}
     dyn = {k: _row_major(_as4(getattr(dynamics, k))).to(dt) for k in DYN_KEYS}
 
-    def per_sample(t, nd):   # gains with an optional leading sample axis -> (S, ...) contiguous
-        if t is None:
-            return None
-        t = t if t.dim() == nd + 1 else t.unsqueeze(0)
-        return t.expand(S, *t.shape[1:]).to(dt).contiguous()
-
     vec = lambda v: None if v is None else torch.as_tensor(v, dtype=dt, device=dev).reshape(-1).contiguous()
-    out = lib.simulate(dims, act, dyn, per_sample(L, 3), per_sample(l, 2), per_sample(K, 3), seed, x0=vec(x0), xhat0=vec(xhat0),
-                       return_all=return_all, stream=_stream(dev), C_noise=C, D_noise=D)   # C, D: signal-dependent-noise extension
-    if actor.A.dim() == 3 and dynamics.A.dim() == 3:
-        return tuple(o[0] for o in out) if return_all else out[0]
-    return out
+    out = lib.simulate(dims, act, dyn, _per_sample(L, 3, S, dt), _per_sample(l, 2, S, dt), _per_sample(K, 3, S, dt), seed,
+                       x0=vec(x0), xhat0=vec(xhat0), return_all=return_all, stream=_stream(dev),
+                       C_noise=C, D_noise=D)   # C, D: signal-dependent-noise extension
+    return _unbatch(actor, dynamics, out)
 
 
 def sdn_log_likelihood(actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, L: torch.Tensor, K: torch.Tensor,
@@ -378,28 +379,17 @@ def sdn_log_likelihood(actor: LQGSpec, dynamics: LQGSpec, x: torch.Tensor, L: to
     _require_cuda(actor.A, "actor spec")
     _require_cuda(x, "observations")
     lib = abi.load_library()
-    per_sample = x.dim() == 4
-    n, T1, d = x.shape[-3:]
-    dims = dims_of(actor, dynamics, n, d)
-    if dims.T != T1 - 1:
-        raise ValueError(f"need T+1 = {dims.T + 1} observations per trial, got {T1}")
-    if per_sample and x.shape[0] != dims.S:
-        raise ValueError(f"per-sample observations need a leading axis of {dims.S} samples, got {x.shape[0]}")
+    dims = dims_of(actor, dynamics, x.shape[-3], x.shape[-1])
     if (dims.x, dims.b, dims.u, dims.y, dims.d) not in FP64_ONLY_DIMS:
         check_supported(dims)
     if dims.x + dims.b > 12:
         raise NotImplementedError("lqg_b200: the signal-dependent-noise / all-FP64 likelihood is compiled for joint dims <= 12")
     dt, dev = actor.A.dtype, actor.A.device
-    act, dyn = _base_mats(actor, dynamics, dt)
-    for M in list(act.values()) + list(dyn.values()):
-        if M.dim() == 4:
-            raise NotImplementedError("lqg_b200: the signal-dependent-noise likelihood needs time-invariant specs")
-    x_tm = x.detach().permute(0, 2, 1, 3).to(torch.float32).contiguous() if per_sample else lib.pack_obs(x.detach(), stream=_stream(dev))
-    S = dims.S
 
-    def per_s(t, nd):
-        t = t if t.dim() == nd + 1 else t.unsqueeze(0)
-        return t.expand(S, *t.shape[1:]).to(dt).contiguous()
-
-    ll = lib.sdn_loglik(dims, act, dyn, per_s(L, 3), per_s(K, 3), x_tm, C_noise=C, D_noise=D, stream=_stream(dev))
-    return ll[0] if (actor.A.dim() == 3 and dynamics.A.dim() == 3) else ll
+    def call(x_tm, act, dyn, s0):
+        for M in list(act.values()) + list(dyn.values()):
+            if M.dim() == 4:
+                raise NotImplementedError("lqg_b200: the signal-dependent-noise likelihood needs time-invariant specs")
+        return lib.sdn_loglik(dims, act, dyn, _per_sample(L, 3, dims.S, dt), _per_sample(K, 3, dims.S, dt), x_tm, C_noise=C,
+                              D_noise=D, stream=_stream(dev))
+    return _observed_call(lib, dims, actor, dynamics, x, None, call)

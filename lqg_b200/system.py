@@ -165,22 +165,7 @@ class System:
         """``simulate`` (system.py:62-140) under signal-dependent noise -- the generative model of ``log_likelihood_sdn``
         (EXTENSION, oracle/sdn_np.py: sdn_simulate): control-dependent process noise ``sum_i eps'_i C_i u_t`` and state-dependent
         observation noise ``sum_j eta'_j D_j x_{t+1}`` on top of V, W.  Arguments as in ``log_likelihood_sdn``; CUDA only."""
-        from lqg_b200.control import sdn
-        if C is None and signal_dep_noise is not None:
-            C = sdn.channel_noise(self, signal_dep_noise, "control")
-        if D is None and obs_dep_noise is not None:
-            D = sdn.channel_noise(self, obs_dep_noise, "observation")
-        if gains is None:
-            g, K = self._gains(Sigma0)
-            L, l = g.L, g.l
-        elif isinstance(gains, str):
-            if gains != "sdn":
-                raise ValueError("gains must be None, 'sdn' or a pair (L, K)")
-            sg = sdn.solve_for_actor(self, signal_dep_noise=signal_dep_noise, obs_dep_noise=obs_dep_noise, Sigma0=Sigma0)
-            L, K = (sg.L, sg.K) if self.actor.A.dim() == 4 else (sg.L[0], sg.K[0])
-            l = None
-        else:
-            (L, K), l = gains, None
+        C, D, L, l, K = self._sdn_inputs(signal_dep_noise, obs_dep_noise, C, D, gains, Sigma0)
         out = runtime.simulate(self.actor, self.dynamics, L, l, K, n, int(rng_key), x0=x0, xhat0=xhat0, return_all=return_all, C=C, D=D)
         if out is None:
             raise NotImplementedError("simulate_sdn: a dimension exceeds the simulator kernel's limit (40)")
@@ -205,7 +190,6 @@ class System:
         matrices ``C[(S,) nc, x, u]``, ``D[(S,) nd, y, x]``.  ``gains``: None = the actor model's own lqr.backward / kf.forward
         (an actor unaware of the multiplicative noise), ``"sdn"`` = the filter-form Todorov iterations on the actor's model with
         the same per-channel scales (lqg_b200.control.sdn.solve_for_actor), or an explicit pair (L, K)."""
-        from lqg_b200.control import sdn
         axis = getattr(self, "_axis_system", None)
         if axis is not None and C is None and D is None and (gains is None or gains == "sdn") and Sigma0 is None and x.shape[-1] == self.xdim:
             # per-channel noise keeps the axes of a dim > 1 tracking model independent: same factorisation as log_likelihood
@@ -214,22 +198,29 @@ class System:
             xa = x.reshape(*lead, n, T1, dim, d // dim).movedim(-2, -4).reshape(*lead, dim * n, T1, d // dim)
             ll = axis.log_likelihood_sdn(xa, signal_dep_noise=signal_dep_noise, obs_dep_noise=obs_dep_noise, gains=gains)
             return ll.reshape(*ll.shape[:-1], dim, n).sum(-2)
+        C, D, L, _, K = self._sdn_inputs(signal_dep_noise, obs_dep_noise, C, D, gains, Sigma0)
+        return runtime.sdn_log_likelihood(self.actor, self.dynamics, x.to(self.device), L, K, C=C, D=D)
+
+    def _sdn_inputs(self, signal_dep_noise, obs_dep_noise, C, D, gains, Sigma0):
+        """(C, D, L, l, K) of simulate_sdn / log_likelihood_sdn: the noise matrices (from the per-channel scales unless given)
+        and the gains named by ``gains``; l is the affine control term of the actor's own gains, None for the others."""
+        from lqg_b200.control import sdn
         if C is None and signal_dep_noise is not None:
             C = sdn.channel_noise(self, signal_dep_noise, "control")
         if D is None and obs_dep_noise is not None:
             D = sdn.channel_noise(self, obs_dep_noise, "observation")
         if gains is None:
             g, K = self._gains(Sigma0)
-            L = g.L
-        elif isinstance(gains, str):
-            if gains != "sdn":
-                raise ValueError("gains must be None, 'sdn' or a pair (L, K)")
-            # the actor plans and filters knowing about the multiplicative noise: filter-form Todorov iterations on its own model
-            sg = sdn.solve_for_actor(self, signal_dep_noise=signal_dep_noise, obs_dep_noise=obs_dep_noise, Sigma0=Sigma0)
-            L, K = (sg.L, sg.K) if self.actor.A.dim() == 4 else (sg.L[0], sg.K[0])
-        else:
+            return C, D, g.L, g.l, K
+        if not isinstance(gains, str):
             L, K = gains
-        return runtime.sdn_log_likelihood(self.actor, self.dynamics, x.to(self.device), L, K, C=C, D=D)
+            return C, D, L, None, K
+        if gains != "sdn":
+            raise ValueError("gains must be None, 'sdn' or a pair (L, K)")
+        # the actor plans and filters knowing about the multiplicative noise: filter-form Todorov iterations on its own model
+        sg = sdn.solve_for_actor(self, signal_dep_noise=signal_dep_noise, obs_dep_noise=obs_dep_noise, Sigma0=Sigma0)
+        L, K = (sg.L, sg.K) if self.actor.A.dim() == 4 else (sg.L[0], sg.K[0])
+        return C, D, L, None, K
 
     # -- slow paths ----------------------------------------------------------------------------------------
     def _joint(self, gains_L, K):

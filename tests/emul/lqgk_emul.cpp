@@ -8,7 +8,7 @@
 
 #include "../../include/lqgk.h"
 #include "../../lqg_b200/csrc/lqgk_core.h"
-#include "../../lqg_b200/csrc/lqgk_dims.h"
+#include "../../lqg_b200/csrc/lqgk_entry.h"
 #include "../../lqg_b200/csrc/lqgk_pack.h"
 #include "../../lqg_b200/csrc/lqgk_stages.h"
 #include "../../lqg_b200/csrc/lqgk_sdn.cuh"
@@ -32,29 +32,26 @@ struct SumSrc {
   float get(int idx) const { return row[idx]; }
 };
 
-static bool time_varying(const LqgkSpec& s) {
-  const LqgkMat* m[] = {&s.A, &s.B, &s.F, &s.V, &s.W, &s.Q, &s.R, &s.q, &s.r, &s.P};
-  for (auto p : m)
-    if (p->ptr && p->time_stride != 0) return true;
-  return false;
-}
-
 template <class DM, class T>
-int run(const LqgkDims& d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkMat* sigma0, const float* x_tm,
-        const T* ll_bar, T* ll_out, const LqgkSpecGrad* gact, const LqgkSpecGrad* gdyn, const LqgkMatGrad* gsig0,
-        bool want_grad, T* L_out, T* l_out, T* H_out, T* K_out, double eps, int mode, T* mu_out = nullptr, T* Sig_out = nullptr) {
-  const int S = d.S, N = d.N, Tn = d.T;
+int run(const Call& c) {
+  const LqgkDims& d = *c.dims;
+  const LqgkSpec *act = c.act, *dyn = c.dyn;
+  const float* x_tm = c.x_tm;
+  const T* ll_bar = (const T*)c.ll_bar;
+  T *ll_out = (T*)c.ll_out, *L_out = (T*)c.L_out, *l_out = (T*)c.l_out, *H_out = (T*)c.H_out, *K_out = (T*)c.K_out;
+  T *mu_out = (T*)c.mu_out, *Sig_out = (T*)c.Sig_out;
+  const int mode = c.mode, S = d.S, N = d.N, Tn = d.T;
+  const bool want_grad = mode == LQGK_MODE_VJP, has_dyn = dyn != nullptr;
   constexpr CLayout cl = DM::CL;
-  const bool has_dyn = dyn != nullptr;
-  const bool tv = time_varying(*act) || (has_dyn && time_varying(*dyn));
-  if (tv && want_grad) return LQGK_E_UNSUPPORTED;
+  const bool tv = spec_time_varying(*act, true) || (has_dyn && spec_time_varying(*dyn, false));
+  if (!kernels_cover(c, tv, DM::N > 12)) return LQGK_E_UNSUPPORTED;
   const size_t Sc = S;
   const size_t tstride = tv ? (size_t)cl.total * Sc : 0;
   std::vector<double> cst((size_t)cl.total * Sc * (tv ? Tn : 1)), acc((size_t)cl.total * Sc, 0.0);
   PackArgs<T> pa{};
   pa.act = *act;
   if (has_dyn) pa.dyn = *dyn;
-  pa.sigma0 = sigma0 ? *sigma0 : LqgkMat{nullptr, 0, 0};
+  pa.sigma0 = c.sigma0 ? *c.sigma0 : LqgkMat{nullptr, 0, 0};
   pa.x = DM::X; pa.b = DM::B; pa.u = DM::U; pa.y = DM::Y; pa.nT = Tn; pa.has_dyn = has_dyn;
   for (int t = 0; t < (tv ? Tn : 1); ++t)
     for (int s = 0; s < S; ++s) {
@@ -75,7 +72,7 @@ int run(const LqgkDims& d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkM
     GCst g{cst.data() + s, Sc, tstride};
     if (mode == LQGK_MODE_GAINS) {
       if (L_out) {
-        lqr_fwd_body<DM, true>(g, WView{lc.data(), 1}, Tn, eps, V(Lw, s), false, V(Sw, s), V(lw, s), V(Hw, s));
+        lqr_fwd_body<DM, true>(g, WView{lc.data(), 1}, Tn, c.eps, V(Lw, s), false, V(Sw, s), V(lw, s), V(Hw, s));
         for (int t = 0; t < Tn; ++t) {
           for (int i = 0; i < DM::EL; ++i) L_out[((size_t)s * Tn + t) * DM::EL + i] = (T)Lw[((size_t)t * DM::EL + i) * Sc + s];
           if (l_out) for (int i = 0; i < DM::U; ++i) l_out[((size_t)s * Tn + t) * DM::U + i] = (T)lw[((size_t)t * DM::U + i) * Sc + s];
@@ -89,7 +86,7 @@ int run(const LqgkDims& d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkM
       }
       continue;
     }
-    lqr_fwd_body<DM, false>(g, WView{lc.data(), 1}, Tn, eps, V(Lw, s), want_grad, V(Sw, s), V(lw, s), V(Hw, s));
+    lqr_fwd_body<DM, false>(g, WView{lc.data(), 1}, Tn, c.eps, V(Lw, s), want_grad, V(Sw, s), V(lw, s), V(Hw, s));
     kf_fwd_body<DM>(g, WView{lc.data(), 1}, Tn, V(Kw, s), want_grad, V(Pw, s));
   }
   if (mode == LQGK_MODE_GAINS) return LQGK_OK;
@@ -178,12 +175,12 @@ int run(const LqgkDims& d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkM
       flush_acc<CovC<DM>>(ga, WView{la.data(), 1}, CovC<DM>::NSEG);
     }
     kf_rev_body<DM>(g, WView{lc.data(), 1}, WView{la.data(), 1}, Tn, V(Pw, s), V(Kbw, s), ga);
-    lqr_rev_body<DM>(g, WView{lc.data(), 1}, WView{la.data(), 1}, Tn, eps, V(Lw, s), V(Sw, s), V(Lbw, s), ga);
+    lqr_rev_body<DM>(g, WView{lc.data(), 1}, WView{la.data(), 1}, Tn, c.eps, V(Lw, s), V(Sw, s), V(Lbw, s), ga);
     UnpackArgs<T> ua{};
     ua.act = *act; ua.dyn = *dyn; ua.sigma0 = pa.sigma0;
-    if (gact) ua.gact = *gact;
-    if (gdyn) ua.gdyn = *gdyn;
-    if (gsig0) ua.gsigma0 = *gsig0;
+    if (c.gact) ua.gact = *c.gact;
+    if (c.gdyn) ua.gdyn = *c.gdyn;
+    if (c.gsig0) ua.gsigma0 = *c.gsig0;
     ua.x = DM::X; ua.b = DM::B; ua.u = DM::U; ua.y = DM::Y;
     WView cv{cst.data() + s, Sc};
     unpack_sample<T>(ua, s, [&](int e) { return (double)ga(e); }, [&](int e) { return (double)cv(e); });
@@ -192,76 +189,43 @@ int run(const LqgkDims& d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkM
 }
 
 template <class T>
-int dispatch(const LqgkDims* d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkMat* sigma0, const float* x_tm,
-             const T* ll_bar, T* ll_out, const LqgkSpecGrad* gact, const LqgkSpecGrad* gdyn, const LqgkMatGrad* gsig0,
-             bool want_grad, T* L_out, T* l_out, T* H_out, T* K_out, double eps, int mode, T* mu_out = nullptr, T* Sig_out = nullptr) {
-  if (!d || !act) return LQGK_E_INVALID;
-#define LQGK_CASE(X, B, U, Y, D)                                                                              \
-  if (d->x == X && d->b == B && d->u == U && d->y == Y && (d->d == D || mode == LQGK_MODE_GAINS))             \
-    return run<Dims<X, B, U, Y, D>, T>(*d, act, dyn, sigma0, x_tm, ll_bar, ll_out, gact, gdyn, gsig0, want_grad, \
-                                       L_out, l_out, H_out, K_out, eps, mode, mu_out, Sig_out);
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return LQGK_E_UNSUPPORTED;
+int dispatch(const Call& c) {
+  if (int rc = validate(c)) return rc;
+  return visit_tuple<Tuples::compiled>(call_key(*c.dims, c.mode), LQGK_E_UNSUPPORTED, [&](auto dm, auto) { return run<decltype(dm), T>(c); });
 }
-}  // namespace
 
 template <class T>
-static int pack_obs_host(int32_t N, int32_t T1, int32_t d, const T* x, float* x_tm) {
+int pack_obs_host(int32_t N, int32_t T1, int32_t d, const T* x, float* x_tm) {
+  if (int rc = check_pack_obs(N, T1, d, x, x_tm)) return rc;
   for (int i = 0; i < N; ++i)
     for (int t = 0; t < T1; ++t)
       for (int k = 0; k < d; ++k) x_tm[((size_t)t * N + i) * d + k] = (float)x[((size_t)i * T1 + t) * d + k];
   return LQGK_OK;
 }
 template <class T>
-static int sdn_loglik_host(const LqgkDims* d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkSdnNoise* nz, const T* L, const T* K,
-                           const float* x_tm, T* ll_out) {
-  if (!d || !act || !dyn || !L || !K || !x_tm || !ll_out) return LQGK_E_INVALID;
-  SdnLikArgs a{};
-  a.act = *act; a.dyn = *dyn; a.L = L; a.K = K; a.x_tm = x_tm; a.x_sample_stride = d->x_sample_stride; a.ll_out = ll_out;
-  a.S = d->S; a.N = d->N; a.T = d->T;
-  if (nz) { a.C = nz->C; a.D = nz->D; a.nc = nz->nc; a.nd = nz->nd; }
-#define LQGK_CASE(X, B, U, Y, DD)                                                                          \
-  if (X + B <= 12 && d->x == X && d->b == B && d->u == U && d->y == Y && d->d == DD) {                     \
-    for (int s = 0; s < a.S; ++s)                                                                          \
-      for (int i = 0; i < a.N; ++i) ll_out[(size_t)s * a.N + i] = (T)SdnLik<Dims<X, B, U, Y, DD>>::template trial<T>(a, s, i); \
-    return LQGK_OK;                                                                                        \
-  }
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-  LQGK_FOR_EACH_FP64_ONLY_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return LQGK_E_UNSUPPORTED;
+int sdn_loglik_host(const LqgkDims* d, const LqgkSpec* act, const LqgkSpec* dyn, const LqgkSdnNoise* nz, const T* L, const T* K,
+                    const float* x_tm, T* ll_out) {
+  SdnLikArgs a;
+  if (int rc = sdn_lik_args(d, act, dyn, nz, L, K, x_tm, ll_out, a)) return rc;
+  return visit_tuple<Tuples::small_and_fp64_only>(full_key(*d), LQGK_E_UNSUPPORTED, [&](auto dm, auto) {
+    for (int s = 0; s < a.S; ++s)
+      for (int i = 0; i < a.N; ++i) ll_out[(size_t)s * a.N + i] = (T)SdnLik<decltype(dm)>::template trial<T>(a, s, i);
+    return LQGK_OK;
+  });
 }
-static int sdn_gains_host(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, int filter_form) {
-  if (!d || !sp || !L_out || !K_out) return LQGK_E_INVALID;
-  SdnArgs a{};
-  auto P = [](const LqgkMat& m) { return (const double*)m.ptr; };
-  a.A = P(sp->A); a.sA = sp->A.sample_stride;
-  a.B = P(sp->B); a.sB = sp->B.sample_stride;
-  a.H = P(sp->H); a.sH = sp->H.sample_stride;
-  a.C = P(sp->C); a.sC = sp->C.sample_stride;
-  a.D = P(sp->D); a.sD = sp->D.sample_stride;
-  a.Q = P(sp->Q); a.sQ = sp->Q.sample_stride;
-  a.R = P(sp->R); a.sR = sp->R.sample_stride;
-  a.Qf = sp->Qf.ptr ? P(sp->Qf) : P(sp->Q); a.sQf = sp->Qf.ptr ? sp->Qf.sample_stride : sp->Q.sample_stride;
-  a.Omxi = P(sp->Om_xi); a.sOmxi = sp->Om_xi.sample_stride;
-  a.Omom = P(sp->Om_omega); a.sOmom = sp->Om_omega.sample_stride;
-  a.Sig1 = P(sp->Sigma1); a.sSig1 = sp->Sigma1.sample_stride;
-  a.xh1 = P(sp->xhat1); a.sxh1 = sp->xhat1.sample_stride;
-  a.S = d->S; a.T = d->T; a.nc = d->nc; a.nd = d->nd; a.sweeps = d->sweeps;
-  a.L = L_out; a.K = K_out; a.cost = cost_out; a.filter_form = filter_form;
-#define LQGK_CASE(X, B, U, Y, DD)                                             \
-  if (X + B <= 12 && d->b == B && d->u == U && d->y == Y) {                   \
-    for (int s = 0; s < a.S; ++s) {                                           \
-      const double c = Sdn<Dims<X, B, U, Y, DD>>::solve(a, s);                \
-      if (cost_out) cost_out[s] = c;                                          \
-    }                                                                         \
-    return LQGK_OK;                                                           \
-  }
-  LQGK_FOR_EACH_DIMS(LQGK_CASE)
-#undef LQGK_CASE
-  return LQGK_E_UNSUPPORTED;
+int sdn_gains_host(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, int filter_form) {
+  SdnArgs a;
+  if (int rc = sdn_gains_args(d, sp, L_out, K_out, cost_out, filter_form, a)) return rc;
+  return visit_tuple<Tuples::small>(TupleKey{ANY, d->b, d->u, d->y, ANY}, LQGK_E_UNSUPPORTED, [&](auto dm, auto) {
+    for (int s = 0; s < a.S; ++s) {
+      const double c = Sdn<decltype(dm)>::solve(a, s);
+      if (cost_out) cost_out[s] = c;
+    }
+    return LQGK_OK;
+  });
 }
+}  // namespace
+
 extern "C" {
 int lqgk_sdn_gains_f64(const LqgkSdnDims* d, const LqgkSdnSpec* sp, double* L_out, double* K_out, double* cost_out, void*) {
   return sdn_gains_host(d, sp, L_out, K_out, cost_out, 0);
@@ -275,47 +239,57 @@ int lqgk_sdn_loglik_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkS
 }
 int lqgk_lqr_backward_f64(const LqgkDims* dims, const LqgkSpec* actor, double eps, double* L_out, double* l_out,
                           double* H_out, void*, size_t, void*) {
-  return dispatch<double>(dims, actor, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, false,
-                          L_out, l_out, H_out, nullptr, eps, LQGK_MODE_GAINS);
+  Call c;
+  c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.eps = eps; c.L_out = L_out; c.l_out = l_out; c.H_out = H_out;
+  return dispatch<double>(c);
 }
 int lqgk_kf_forward_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double* K_out, void*,
                         size_t, void*) {
-  return dispatch<double>(dims, actor, nullptr, sigma0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, false,
-                          nullptr, nullptr, nullptr, K_out, 1e-8, LQGK_MODE_GAINS);
+  Call c;
+  c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.sigma0 = sigma0; c.K_out = K_out;
+  return dispatch<double>(c);
 }
 int lqgk_loglik_fwd_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, double* ll_out, void*, size_t, void*) {
-  return dispatch<double>(dims, actor, dynamics, sigma0, x_tm, nullptr, ll_out, nullptr, nullptr, nullptr, false,
-                          nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_FWD);
+  Call c;
+  c.mode = LQGK_MODE_FWD; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_out = ll_out;
+  return dispatch<double>(c);
 }
 int lqgk_loglik_vjp_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, const double* ll_bar, double* ll_out, const LqgkSpecGrad* ga,
                         const LqgkSpecGrad* gd, const LqgkMatGrad* gs, void*, size_t, void*) {
-  return dispatch<double>(dims, actor, dynamics, sigma0, x_tm, ll_bar, ll_out, ga, gd, gs, true, nullptr, nullptr,
-                          nullptr, nullptr, 1e-8, LQGK_MODE_VJP);
+  Call c;
+  c.mode = LQGK_MODE_VJP; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_bar = ll_bar;
+  c.ll_out = ll_out; c.gact = ga; c.gdyn = gd; c.gsig0 = gs;
+  return dispatch<double>(c);
 }
 int lqgk_loglik_fwd_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, float* ll_out, void*, size_t, void*) {
-  return dispatch<float>(dims, actor, dynamics, sigma0, x_tm, nullptr, ll_out, nullptr, nullptr, nullptr, false,
-                         nullptr, nullptr, nullptr, nullptr, 1e-8, LQGK_MODE_FWD);
+  Call c;
+  c.mode = LQGK_MODE_FWD; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_out = ll_out;
+  return dispatch<float>(c);
 }
 int lqgk_loglik_vjp_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, const float* ll_bar, float* ll_out, const LqgkSpecGrad* ga,
                         const LqgkSpecGrad* gd, const LqgkMatGrad* gs, void*, size_t, void*) {
-  return dispatch<float>(dims, actor, dynamics, sigma0, x_tm, ll_bar, ll_out, ga, gd, gs, true, nullptr, nullptr,
-                         nullptr, nullptr, 1e-8, LQGK_MODE_VJP);
+  Call c;
+  c.mode = LQGK_MODE_VJP; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.ll_bar = ll_bar;
+  c.ll_out = ll_out; c.gact = ga; c.gdyn = gd; c.gsig0 = gs;
+  return dispatch<float>(c);
 }
 int lqgk_moments_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0, const float* x_tm,
                      double* mu_out, double* Sigma_out, void*, size_t, void*) {
-  if (dims && dims->x + dims->b > 12) return LQGK_E_UNSUPPORTED;
-  return dispatch<double>(dims, actor, dynamics, sigma0, x_tm, nullptr, nullptr, nullptr, nullptr, nullptr, false, nullptr, nullptr,
-                          nullptr, nullptr, 1e-8, LQGK_MODE_MOMENTS, mu_out, Sigma_out);
+  Call c;
+  c.mode = LQGK_MODE_MOMENTS; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.mu_out = mu_out;
+  c.Sig_out = Sigma_out;
+  return dispatch<double>(c);
 }
 int lqgk_moments_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0, const float* x_tm,
                      float* mu_out, float* Sigma_out, void*, size_t, void*) {
-  if (dims && dims->x + dims->b > 12) return LQGK_E_UNSUPPORTED;
-  return dispatch<float>(dims, actor, dynamics, sigma0, x_tm, nullptr, nullptr, nullptr, nullptr, nullptr, false, nullptr, nullptr,
-                         nullptr, nullptr, 1e-8, LQGK_MODE_MOMENTS, mu_out, Sigma_out);
+  Call c;
+  c.mode = LQGK_MODE_MOMENTS; c.dims = dims; c.act = actor; c.dyn = dynamics; c.sigma0 = sigma0; c.x_tm = x_tm; c.mu_out = mu_out;
+  c.Sig_out = Sigma_out;
+  return dispatch<float>(c);
 }
 int lqgk_pack_obs_f32(int32_t N, int32_t T1, int32_t d, const float* x, float* x_tm, void*) { return pack_obs_host(N, T1, d, x, x_tm); }
 int lqgk_pack_obs_f64(int32_t N, int32_t T1, int32_t d, const double* x, float* x_tm, void*) { return pack_obs_host(N, T1, d, x, x_tm); }
