@@ -79,7 +79,7 @@ typedef struct {
  * lqgk_kf_forward_*:   replaces lqg/belief/kf.py:6-21     kf.forward(spec, Sigma0) -> K.
  *   sigma0: [b][b] per sample (time_stride ignored); absent -> V[0] V[0]^T (lqg/system.py:158-161).
  *   Output K[S][T][b][y].
- * `d` in dims is ignored by the gains entry points (set it to any supported value, e.g. min(x, 2)).    */
+ * `d` and `N` in dims are ignored by the gains entry points and their adjoint (set d to any supported value, e.g. min(x, 2)). */
 int lqgk_lqr_backward_f32(const LqgkDims* dims, const LqgkSpec* actor, double eps, float* L_out, float* l_out,
                           float* H_out, void* workspace, size_t workspace_bytes, void* stream);
 int lqgk_lqr_backward_f64(const LqgkDims* dims, const LqgkSpec* actor, double eps, double* L_out, double* l_out,
@@ -88,6 +88,22 @@ int lqgk_kf_forward_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkM
                         void* workspace, size_t workspace_bytes, void* stream);
 int lqgk_kf_forward_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double* K_out,
                         void* workspace, size_t workspace_bytes, void* stream);
+/* lqgk_gains_vjp_*: reverse-mode adjoint of the two sweeps above (what jax.vjp of lqr.backward(spec, eps).L and of
+ *   kf.forward(spec, Sigma0) computes in the reference).  L_bar[S][T][u][b] and K_bar[S][T][b][y] are the cotangents of L and
+ *   K in the layouts of those outputs; either may be NULL (zero), not both.  eps and sigma0 as above.  The call recomputes
+ *   both sweeps and keeps S_t / P_t in the workspace (no state from an earlier call), then runs the Riccati and Kalman
+ *   adjoints; the eigen-shift of lqr.py:27-28 is held constant, as in lqgk_loglik_vjp_*.
+ *   actor_grad receives the gradients of A, B, F, V, W, Q, R, Qf (any field may be NULL), sigma0_grad that of Sigma0 (may be
+ *   NULL).  Defaulted inputs send their gradient to their source: Qf absent -> Q; sigma0 absent -> actor V.
+ *   A, B, F, V, W, Q, R are required.  The affine terms q, r, qf are not read (L and K do not depend on them); a cross cost P
+ *   and time-varying specs -> LQGK_E_UNSUPPORTED.  Workspace: lqgk_workspace_bytes(dims, LQGK_MODE_GAINS_VJP, max_chunk).
+ *   Runs on `stream` alone (never on the internal streams), so it can be captured into a CUDA graph.                      */
+int lqgk_gains_vjp_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double eps, const float* L_bar,
+                       const float* K_bar, const LqgkSpecGrad* actor_grad, const LqgkMatGrad* sigma0_grad, void* workspace,
+                       size_t workspace_bytes, void* stream);
+int lqgk_gains_vjp_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double eps, const double* L_bar,
+                       const double* K_bar, const LqgkSpecGrad* actor_grad, const LqgkMatGrad* sigma0_grad, void* workspace,
+                       size_t workspace_bytes, void* stream);
 
 /* ---- likelihood ---------------------------------------------------------------------------------------
  * lqgk_loglik_fwd_*: replaces lqg/system.py:142-248  System.log_likelihood(x) (= conditional_moments +
@@ -194,6 +210,7 @@ int lqgk_pack_obs_f64(int32_t N, int32_t T1, int32_t d, const double* x, float* 
 #define LQGK_MODE_FWD 1
 #define LQGK_MODE_VJP 2
 #define LQGK_MODE_MOMENTS 3
+#define LQGK_MODE_GAINS_VJP 4
 /* Bytes of workspace that let `mode` process min(S, max_chunk) samples per internal chunk (max_chunk <= 0:
  * all S at once).  Any size >= lqgk_workspace_bytes(dims, mode, 32) is accepted; larger = fewer chunks.   */
 size_t lqgk_workspace_bytes(const LqgkDims* dims, int mode, int32_t max_chunk);

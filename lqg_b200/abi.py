@@ -17,7 +17,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("LQGK_LIB_PATH") or os.path.join(HERE, "csrc", "liblqgk.so")   # override: tuning experiments (tools/)
 
-MODE_GAINS, MODE_FWD, MODE_VJP, MODE_MOMENTS = 0, 1, 2, 3
+MODE_GAINS, MODE_FWD, MODE_VJP, MODE_MOMENTS, MODE_GAINS_VJP = 0, 1, 2, 3, 4
 ACTOR_KEYS = ("A", "B", "F", "V", "W", "Q", "R")
 DYN_KEYS = ("A", "B", "F", "V", "W")
 
@@ -184,6 +184,36 @@ class Library:
         self._check(fn(C.byref(dims), C.byref(sp), C.byref(s0) if s0 is not None else None,
                        C.c_void_p(K.data_ptr()), C.c_void_p(p), C.c_size_t(n), C.c_void_p(stream)), "lqgk_kf_forward")
         return K
+
+    def gains_vjp(self, dims, actor, sigma0=None, eps=1e-8, L_bar=None, K_bar=None, want=ACTOR_KEYS, ws=None, stream=0):
+        """Gradients of <L_bar, L> + <K_bar, K> (lqr_backward's L, kf_forward's K; either cotangent may be None, not both)
+        with respect to the actor's base matrices: ({name: [S, r, c]} for the names in `want` -- ACTOR_KEYS and "Qf" --, the
+        gradient of sigma0 [S, b, b] or None).  actor: time-invariant base matrices as for loglik_vjp."""
+        dt, dev = actor["A"].dtype, actor["A"].device
+        S, T = dims.S, dims.T
+        sp = self._spec(actor, S, T, ACTOR_KEYS)
+        s0 = _mat(sigma0, S, 1) if sigma0 is not None else None
+        shp = dict(A=(dims.b, dims.b), B=(dims.b, dims.u), F=(dims.y, dims.b), V=(dims.b, dims.b), W=(dims.y, dims.y),
+                   Q=(dims.b, dims.b), R=(dims.u, dims.u), Qf=(dims.b, dims.b))
+        ga, out = LqgkSpecGrad(), {}
+        for k in want:
+            out[k] = torch.empty((S,) + shp[k], dtype=dt, device=dev)
+            setattr(ga, k, LqgkMatGrad(out[k].data_ptr(), out[k].stride(0)))
+        gs0, out_s0 = None, None
+        if sigma0 is not None:
+            out_s0 = torch.empty((S, dims.b, dims.b), dtype=dt, device=dev)
+            gs0 = LqgkMatGrad(out_s0.data_ptr(), out_s0.stride(0))
+        keep = [None if v is None else v.to(dt).contiguous() for v in (L_bar, K_bar)]
+        for v, shape in zip(keep, ((S, T, dims.u, dims.b), (S, T, dims.b, dims.y))):
+            assert v is None or tuple(v.shape) == shape, (tuple(v.shape), shape)
+        p, n = self._ws(ws)
+        fn = getattr(self.lib, "lqgk_gains_vjp_" + self._suffix(dt))
+        self._check(fn(C.byref(dims), C.byref(sp), C.byref(s0) if s0 is not None else None, C.c_double(eps),
+                       C.c_void_p(keep[0].data_ptr() if keep[0] is not None else None),
+                       C.c_void_p(keep[1].data_ptr() if keep[1] is not None else None), C.byref(ga),
+                       C.byref(gs0) if gs0 is not None else None, C.c_void_p(p), C.c_size_t(n), C.c_void_p(stream)),
+                    "lqgk_gains_vjp")
+        return out, out_s0
 
     def loglik_fwd(self, dims, actor, dyn, x_tm, sigma0=None, ws=None, stream=0):
         dt, dev = actor["A"].dtype, actor["A"].device

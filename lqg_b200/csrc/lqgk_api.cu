@@ -247,6 +247,18 @@ int lqgk_kf_forward_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkM
   c.mode = LQGK_MODE_GAINS; c.dims = dims; c.act = actor; c.sigma0 = sigma0; c.K_out = K_out;
   return dispatch<double>(c, ws, ws_bytes, stream);
 }
+int lqgk_gains_vjp_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double eps, const float* L_bar,
+                       const float* K_bar, const LqgkSpecGrad* ga, const LqgkMatGrad* gs, void* ws, size_t ws_bytes, void* stream) {
+  LqgkSpec base;
+  Call c = gains_vjp_call(dims, actor, sigma0, eps, L_bar, K_bar, ga, gs, base);
+  return dispatch<float>(c, ws, ws_bytes, stream);
+}
+int lqgk_gains_vjp_f64(const LqgkDims* dims, const LqgkSpec* actor, const LqgkMat* sigma0, double eps, const double* L_bar,
+                       const double* K_bar, const LqgkSpecGrad* ga, const LqgkMatGrad* gs, void* ws, size_t ws_bytes, void* stream) {
+  LqgkSpec base;
+  Call c = gains_vjp_call(dims, actor, sigma0, eps, L_bar, K_bar, ga, gs, base);
+  return dispatch<double>(c, ws, ws_bytes, stream);
+}
 int lqgk_loglik_fwd_f32(const LqgkDims* dims, const LqgkSpec* actor, const LqgkSpec* dynamics, const LqgkMat* sigma0,
                         const float* x_tm, float* ll_out, void* ws, size_t ws_bytes, void* stream) {
   Call c;
@@ -331,7 +343,7 @@ const char* lqgk_strerror(int code) {
   switch (code) {
     case LQGK_OK: return "ok";
     case LQGK_E_INVALID: return "invalid argument (null pointer, non-positive dimension or misaligned buffer)";
-    case LQGK_E_UNSUPPORTED: return "unsupported: dimension tuple not compiled in, or time-varying spec passed to the VJP";
+    case LQGK_E_UNSUPPORTED: return "unsupported: dimension tuple not compiled in, or time-varying spec (or cross cost P) passed to an adjoint";
     case LQGK_E_WORKSPACE: return "workspace too small for one 32-sample chunk (see lqgk_workspace_bytes)";
     case LQGK_E_CUDA: return "CUDA runtime error";
     case LQGK_E_NOT_INITIALISED: return "internal streams missing while the caller's stream is being captured: call lqgk_init() on this thread and device before capturing";

@@ -19,6 +19,7 @@ struct Call {
   const LqgkMat* sigma0 = nullptr;
   const float* x_tm = nullptr;
   const void* ll_bar = nullptr;
+  const void *L_bar = nullptr, *K_bar = nullptr;   // cotangents of the gains (gains adjoint)
   const LqgkSpecGrad *gact = nullptr, *gdyn = nullptr;
   const LqgkMatGrad* gsig0 = nullptr;
   void *ll_out = nullptr, *L_out = nullptr, *l_out = nullptr, *H_out = nullptr, *K_out = nullptr, *mu_out = nullptr, *Sig_out = nullptr;
@@ -42,13 +43,22 @@ inline int need_closed_loop(const LqgkSpec& act, const LqgkSpec& dyn, bool time_
   return need({&act.A, &act.B, &act.F, &dyn.A, &dyn.B, &dyn.F, &dyn.V, &dyn.W}, time_invariant);
 }
 
+// the modes that run the gain sweeps alone (no observations, no dynamics spec)
+inline bool gains_mode(int mode) { return mode == LQGK_MODE_GAINS || mode == LQGK_MODE_GAINS_VJP; }
+
 inline int validate(const Call& c) {
   if (!c.dims || !c.act) return LQGK_E_INVALID;
   const LqgkDims& d = *c.dims;
   if (d.S <= 0 || d.T <= 0 || d.x <= 0 || d.b <= 0 || d.u <= 0 || d.y <= 0) return LQGK_E_INVALID;
   if (!c.act->A.ptr || !c.act->B.ptr) return LQGK_E_INVALID;
   if (c.mode == LQGK_MODE_GAINS && !c.L_out && !c.K_out) return LQGK_E_INVALID;
-  if (c.mode != LQGK_MODE_GAINS) {
+  if (c.mode == LQGK_MODE_GAINS_VJP) {
+    if (!c.L_bar && !c.K_bar) return LQGK_E_INVALID;
+    const LqgkSpec& a = *c.act;
+    if (need({&a.F, &a.V, &a.W, &a.Q, &a.R})) return LQGK_E_INVALID;
+    if (a.P.ptr) return LQGK_E_UNSUPPORTED;   // the Riccati adjoint has no cross-cost term
+  }
+  if (!gains_mode(c.mode)) {
     if (d.N <= 0 || d.d <= 0 || d.d > d.x) return LQGK_E_INVALID;
     if (!c.dyn || !c.x_tm) return LQGK_E_INVALID;
     if (c.mode == LQGK_MODE_MOMENTS ? (!c.mu_out && !c.Sig_out) : !c.ll_out) return LQGK_E_INVALID;
@@ -70,11 +80,26 @@ inline bool spec_time_varying(const LqgkSpec& s, bool actor) {
     if (m[i]->ptr && m[i]->time_stride != 0) return true;
   return false;
 }
-// What the kernels of a tuple leave out (tv: a time-varying spec; big: joint dim > 12): the adjoint of a time-varying spec,
+// What the kernels of a tuple leave out (tv: a time-varying spec; big: joint dim > 12): the adjoints of a time-varying spec,
 // and for large systems time-varying specs and the predictive moments.
 inline bool kernels_cover(const Call& c, bool tv, bool big) {
-  if (tv && c.mode == LQGK_MODE_VJP) return false;
+  if (tv && (c.mode == LQGK_MODE_VJP || c.mode == LQGK_MODE_GAINS_VJP)) return false;
   return !(big && (tv || c.mode == LQGK_MODE_MOMENTS));
+}
+
+// The gains adjoint (lqgk_gains_vjp_*): `base` receives the actor spec without its affine terms q, r, qf, which the gains do
+// not depend on, so that neither their presence nor a time axis of theirs matters.
+inline Call gains_vjp_call(const LqgkDims* dims, const LqgkSpec* act, const LqgkMat* sigma0, double eps, const void* L_bar,
+                           const void* K_bar, const LqgkSpecGrad* ga, const LqgkMatGrad* gs, LqgkSpec& base) {
+  Call c;
+  c.mode = LQGK_MODE_GAINS_VJP; c.dims = dims; c.sigma0 = sigma0; c.eps = eps; c.L_bar = L_bar; c.K_bar = K_bar; c.gact = ga;
+  c.gsig0 = gs;
+  if (act) {
+    base = *act;
+    base.q = base.r = base.qf = LqgkMat{nullptr, 0, 0};
+    c.act = &base;
+  }
+  return c;
 }
 
 inline int check_pack_obs(int32_t N, int32_t T1, int32_t d, const void* x, const float* x_tm) {
@@ -126,7 +151,7 @@ struct TupleKey {
 };
 inline TupleKey full_key(const LqgkDims& d) { return {d.x, d.b, d.u, d.y, d.d}; }
 // the gains sweeps do not read the observations: their d is any tuple's
-inline TupleKey call_key(const LqgkDims& d, int mode) { return {d.x, d.b, d.u, d.y, mode == LQGK_MODE_GAINS ? ANY : d.d}; }
+inline TupleKey call_key(const LqgkDims& d, int mode) { return {d.x, d.b, d.u, d.y, gains_mode(mode) ? ANY : d.d}; }
 
 enum class Tuples {
   compiled,              // every line of LQGK_FOR_EACH_DIMS

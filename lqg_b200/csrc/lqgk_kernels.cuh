@@ -87,6 +87,14 @@ __global__ void k_unpack(UnpackArgs<T> a, int s0, int n_valid, const double* acc
   unpack_sample<T>(a, s0 + i, [&](int e) { return acc[(size_t)e * Sc + i]; }, [&](int e) { return cst[(size_t)e * Sc + i]; });
 }
 
+// (k_unpack for the gains adjoint, which has no dynamics spec)
+template <class T>
+__global__ void k_unpack_actor(UnpackArgs<T> a, int s0, int n_valid, const double* acc, const double* cst, size_t Sc) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_valid) return;
+  unpack_sample<T, false>(a, s0 + i, [&](int e) { return acc[(size_t)e * Sc + i]; }, [&](int e) { return cst[(size_t)e * Sc + i]; });
+}
+
 // SoA workspace [t][E][Sc] -> user layout [s][t][E]
 template <class T>
 __global__ void k_store_rows(const double* ws, size_t Sc, int n_valid, int Tn, int E, T* out /* already offset by s0 */) {
@@ -97,6 +105,19 @@ __global__ void k_store_rows(const double* ws, size_t Sc, int n_valid, int Tn, i
   int t = (idx / E) % Tn;
   int s = idx / ((size_t)E * Tn);
   out[idx] = (T)ws[((size_t)t * E + e) * Sc + s];
+}
+// The reverse of k_store_rows / k_store_ll for the cotangents of the gains: user layout [s][t][E] -> FP64 workspace, sample-minor
+// [t][E][Sc] (small systems) or sample-major [s][t][E] (large systems); the padded samples n_valid <= s < n_pad get zeros.
+template <class T>
+__global__ void k_load_rows(const T* in /* already offset by s0 */, size_t Sc, int n_valid, int n_pad, int Tn, int E, bool sample_minor,
+                            double* ws) {
+  size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t total = (size_t)n_pad * Tn * E;
+  if (idx >= total) return;
+  int e = idx % E;
+  int t = (idx / E) % Tn;
+  int s = idx / ((size_t)E * Tn);
+  ws[sample_minor ? ((size_t)t * E + e) * Sc + s : idx] = s < n_valid ? (double)in[idx] : 0.0;
 }
 template <class T>
 __global__ void k_store_ll(const double* ll_ws, size_t count, T* out) {

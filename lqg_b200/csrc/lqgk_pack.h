@@ -136,8 +136,9 @@ LQGK_HD void store_grad(const LqgkMatGrad& g, int s, int idx, double v) {
   ((T*)g.ptr)[(int64_t)s * g.sample_stride + idx] = (T)v;
 }
 
-// acc(e): accumulated cotangent of derived constant e; cst(e): the derived constants themselves.
-template <class T, class Acc, class Cst>
+// acc(e): accumulated cotangent of derived constant e; cst(e): the derived constants themselves.  DYN = false: a call
+// without a dynamics spec (the gains adjoint), whose a.dyn is empty: the actor's gradients only.
+template <class T, bool DYN = true, class Acc, class Cst>
 LQGK_HD void unpack_sample(const UnpackArgs<T>& a, int s, Acc&& acc, Cst&& cst) {
   const CLayout cl(a.x, a.b, a.u, a.y);
   const int x = a.x, b = a.b, u = a.u, y = a.y;
@@ -204,6 +205,7 @@ LQGK_HD void unpack_sample(const UnpackArgs<T>& a, int s, Acc&& acc, Cst&& cst) 
   if (a.gsigma0.ptr)
     for (int i = 0; i < b; ++i)
       for (int j = 0; j < b; ++j) store_grad<T>(a.gsigma0, s, i * b + j, a.sigma0.ptr ? acc(cl.Sig0 + sidx(i, j)) : 0.0);
+  if constexpr (!DYN) return;
   // ---- dynamics
   if (a.gdyn.A.ptr)
     for (int i = 0; i < x; ++i)

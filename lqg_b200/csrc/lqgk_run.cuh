@@ -171,6 +171,14 @@ Plan make_plan(const LqgkDims& d, int mode, bool tv, size_t Sc) {
     p.H = take(sizeof(double) * T * DM::U * DM::U * Sc);
   } else if (mode == LQGK_MODE_MOMENTS) {
     p.rec = take(sizeof(float) * Sc * T * DM::REC);
+  } else if (mode == LQGK_MODE_GAINS_VJP) {
+    p.acc = take(sizeof(double) * cl.total * Sc);
+    p.Sric = take(sizeof(double) * T * DM::ES * Sc);
+    p.Pkf = take(sizeof(double) * T * DM::EP * Sc);
+    p.Lbar = take(sizeof(double) * T * DM::EL * Sc);
+    p.Kbar = take(sizeof(double) * T * DM::EK * Sc);
+    p.KbarF = take(sizeof(double) * T * DM::EK * Sc);
+    p.carP = take(sizeof(double) * DM::B * DM::B * Sc);
   } else {
     p.rec = take(sizeof(float) * Sc * T * DM::REC);
     p.ll = take(sizeof(double) * Sc * N);
@@ -289,7 +297,9 @@ struct Chunk {
   size_t s0;                // first sample of the chunk
   int n, npad, nblk, wblk;  // samples (valid, padded to 32); CTAs of the thread- and of the warp-per-sample kernels
   int Tn, N;
-  bool tv, vjp;
+  bool tv;
+  bool vjp;                 // the likelihood's adjoint: its buffers (covariance linearisation points, checkpoints, weights)
+  bool keep;                // keep S_t and P_t for an adjoint (the likelihood's or the gains')
   bool warp_cov;            // covariance kernels one warp per sample (always for the large systems)
   size_t xcs = 0;           // element stride between the repacked observation sets in xc (repack_obs)
 
@@ -309,41 +319,41 @@ struct Chunk {
     LQGK_LAUNCH_CHECK();
     return LQGK_OK;
   }
-  // Riccati sweep, t down.  AFFINE (gains entry point): also l_t and H_t.  VJP: keeps S_t for the adjoint.
+  // Riccati sweep, t down.  AFFINE (gains entry point): also l_t and H_t.  keep: keeps S_t for the adjoint.
   template <bool AFFINE>
   int lqr_fwd(cudaStream_t st) const {
-    double *Sric = vjp ? D(p.Sric) : nullptr, *l = AFFINE ? D(p.l) : nullptr, *H = AFFINE ? D(p.H) : nullptr;
+    double *Sric = keep ? D(p.Sric) : nullptr, *l = AFFINE ? D(p.l) : nullptr, *H = AFFINE ? D(p.H) : nullptr;
     int rc;
     if constexpr (BIG) {
       const size_t smem = BigG<DM>::smem_lqr();
       if ((rc = set_smem<DM>((const void*)kw_lqr_fwd<DM, AFFINE>, smem))) return rc;
       ProfScope ps_(PK_LQR_FWD, st);
-      kw_lqr_fwd<DM, AFFINE><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, c.eps, D(p.L), vjp, Sric, l, H);
+      kw_lqr_fwd<DM, AFFINE><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, c.eps, D(p.L), keep, Sric, l, H);
       LQGK_LAUNCH_CHECK();
     } else {
       const size_t smem = sizeof(double) * 32 * (AFFINE ? LqrC<DM>::n_affine : LqrC<DM>::n);
       if ((rc = set_smem<DM>((const void*)k_lqr_fwd<DM, AFFINE>, smem))) return rc;
       ProfScope ps_(PK_LQR_FWD, st);
-      k_lqr_fwd<DM, AFFINE><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, c.eps, D(p.L), vjp, Sric, l, H);
+      k_lqr_fwd<DM, AFFINE><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, c.eps, D(p.L), keep, Sric, l, H);
       LQGK_LAUNCH_CHECK();
     }
     return LQGK_OK;
   }
-  // Kalman sweep, t up over [t0, t1).  VJP: keeps P_t for the adjoint.
+  // Kalman sweep, t up over [t0, t1).  keep: keeps P_t for the adjoint.
   int kf_fwd(cudaStream_t st, int t0, int t1) const {
-    double* Pkf = vjp ? D(p.Pkf) : nullptr;
+    double* Pkf = keep ? D(p.Pkf) : nullptr;
     int rc;
     if constexpr (BIG) {
       const size_t smem = BigG<DM>::smem_kf();
       if ((rc = set_smem<DM>((const void*)kw_kf_fwd<DM>, smem))) return rc;
       ProfScope ps_(PK_KF_FWD, st);
-      kw_kf_fwd<DM><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, D(p.K), vjp, Pkf);
+      kw_kf_fwd<DM><<<wblk, WTHR, smem, st>>>(D(p.cst), p.Sc, npad, Tn, D(p.K), keep, Pkf);
       LQGK_LAUNCH_CHECK();
     } else {
       const size_t smem = sizeof(double) * 32 * KfC<DM>::n;
       if ((rc = set_smem<DM>((const void*)k_kf_fwd<DM>, smem))) return rc;
       ProfScope ps_(PK_KF_FWD, st);
-      k_kf_fwd<DM><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, D(p.K), vjp, Pkf, t0, t1);
+      k_kf_fwd<DM><<<nblk, 32, smem, st>>>(D(p.cst), p.Sc, tstride(), Tn, D(p.K), keep, Pkf, t0, t1);
       LQGK_LAUNCH_CHECK();
     }
     return LQGK_OK;
@@ -411,11 +421,11 @@ struct Chunk {
     if ((rc = load_w(c.ll_bar ? (const T*)c.ll_bar + s0 * N : nullptr, 0, total))) return rc;
     return padded > total ? load_w(nullptr, total, padded - total) : LQGK_OK;
   }
-  // Zeroes the cotangent accumulators, and the per-step sums of the padded samples: k_trial_rev never writes those, and the
-  // covariance adjoint must read finite data.
+  // Zeroes the cotangent accumulators, and (likelihood adjoint) the per-step sums of the padded samples: k_trial_rev never
+  // writes those, and the covariance adjoint must read finite data.
   int zero_acc(cudaStream_t st) const {
     if (cudaMemsetAsync(D(p.acc), 0, sizeof(double) * DM::CL.total * p.Sc, st) != cudaSuccess) return LQGK_E_CUDA;
-    if (npad > n &&
+    if (vjp && npad > n &&
         cudaMemsetAsync(F(p.sums) + (size_t)n * Tn * DM::SUMP, 0, sizeof(float) * (size_t)(npad - n) * Tn * DM::SUMP, st) != cudaSuccess)
       return LQGK_E_CUDA;
     return LQGK_OK;
@@ -518,16 +528,27 @@ struct Chunk {
     }
     return LQGK_OK;
   }
-  // Cotangent accumulators -> the caller's gradient structs.
+  // Cotangent accumulators -> the caller's gradient structs (the actor's only when the call has no dynamics spec).
   int unpack(cudaStream_t st) const {
     UnpackArgs<T> ua{};
-    ua.act = *c.act; ua.dyn = *c.dyn; ua.sigma0 = c.sigma0 ? *c.sigma0 : LqgkMat{nullptr, 0, 0};
+    ua.act = *c.act; ua.sigma0 = c.sigma0 ? *c.sigma0 : LqgkMat{nullptr, 0, 0};
+    if (c.dyn) ua.dyn = *c.dyn;
     if (c.gact) ua.gact = *c.gact;
     if (c.gdyn) ua.gdyn = *c.gdyn;
     if (c.gsig0) ua.gsigma0 = *c.gsig0;
     ua.x = DM::X; ua.b = DM::B; ua.u = DM::U; ua.y = DM::Y;
     ProfScope ps_(PK_UNPACK, st);
-    k_unpack<T><<<(n + 63) / 64, 64, 0, st>>>(ua, (int)s0, n, D(p.acc), D(p.cst), p.Sc);
+    if (c.dyn) k_unpack<T><<<(n + 63) / 64, 64, 0, st>>>(ua, (int)s0, n, D(p.acc), D(p.cst), p.Sc);
+    else k_unpack_actor<T><<<(n + 63) / 64, 64, 0, st>>>(ua, (int)s0, n, D(p.acc), D(p.cst), p.Sc);
+    LQGK_LAUNCH_CHECK();
+    return LQGK_OK;
+  }
+  // The caller's cotangents of the gains [s][t][E] -> the workspace array at `off` that the matching adjoint sweep reads
+  // (sample-minor for the small systems, sample-major for the large ones).
+  int load_gains_bar(cudaStream_t st, size_t off, int E, const void* in) const {
+    const size_t total = (size_t)npad * Tn * E;
+    ProfScope ps_(PK_MISC, st);
+    k_load_rows<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>((const T*)in + s0 * Tn * E, p.Sc, n, npad, Tn, E, !BIG, D(off));
     LQGK_LAUNCH_CHECK();
     return LQGK_OK;
   }
@@ -576,7 +597,7 @@ int run(const Call& c) {
   if (!kernels_cover(c, tv, is_big<DM>())) return LQGK_E_UNSUPPORTED;
   if (!c.ws || ((uintptr_t)c.ws % ALIGN) != 0) return LQGK_E_INVALID;
   // slices: ns concurrent streams, each with its own workspace part and chunk size Sc
-  int ns = c.mode == LQGK_MODE_GAINS ? 1 : std::max(1, std::min(g_streams, (int)((d.S + 31) / 32)));
+  int ns = gains_mode(c.mode) ? 1 : std::max(1, std::min(g_streams, (int)((d.S + 31) / 32)));
   size_t Sc = 0;
   for (; ns >= 1; --ns) {
     const int32_t want = (int32_t)up(((size_t)d.S + ns - 1) / ns, 32);
@@ -653,7 +674,8 @@ int run(const Call& c) {
       base += (size_t)(chunk_idx % ns) * slice_bytes;
     }
     const bool warp_cov = is_big<DM>() || (!tv && d.S <= g_warp_cov_max_samples);
-    Chunk<DM, T> k{c, p, base, s0, n, npad, npad / 32, (npad + BW_WARPS - 1) / BW_WARPS, Tn, N, tv, vjp, warp_cov};
+    const bool keep = vjp || c.mode == LQGK_MODE_GAINS_VJP;
+    Chunk<DM, T> k{c, p, base, s0, n, npad, npad / 32, (npad + BW_WARPS - 1) / BW_WARPS, Tn, N, tv, vjp, keep, warp_cov};
     int rc;
     if ((rc = k.pack(st))) return rc;
     if (c.mode == LQGK_MODE_GAINS) {
@@ -667,6 +689,24 @@ int run(const Call& c) {
         if ((rc = k.kf_fwd(st, 0, Tn))) return rc;
         if ((rc = k.store_gains(st, p.K, DM::EK, c.K_out))) return rc;
       }
+      continue;
+    }
+    if (c.mode == LQGK_MODE_GAINS_VJP) {
+      // both sweeps again, keeping S_t / P_t, then their adjoints from the caller's cotangents; a NULL cotangent skips its pair
+      if ((rc = k.zero_acc(st))) return rc;
+      if (c.L_bar) {
+        if ((rc = k.template lqr_fwd<false>(st))) return rc;
+        if ((rc = k.load_gains_bar(st, p.Lbar, DM::EL, c.L_bar))) return rc;
+        if ((rc = k.lqr_rev(st))) return rc;
+      }
+      if (c.K_bar) {
+        if ((rc = k.kf_fwd(st, 0, Tn))) return rc;
+        if ((rc = k.load_gains_bar(st, p.Kbar, DM::EK, c.K_bar))) return rc;
+        // the Kalman adjoint of the small systems adds a second cotangent part, which only the likelihood's contraction fills
+        if (!is_big<DM>() && cudaMemsetAsync(k.D(p.KbarF), 0, sizeof(double) * Tn * DM::EK * p.Sc, st) != cudaSuccess) return LQGK_E_CUDA;
+        if ((rc = k.kf_rev(st, 0, Tn))) return rc;
+      }
+      if ((rc = k.unpack(st))) return rc;
       continue;
     }
     if (c.mode == LQGK_MODE_MOMENTS) {

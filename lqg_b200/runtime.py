@@ -162,8 +162,71 @@ def _gains_call(spec: LQGSpec):
     return lib, dims, spec_mats(spec, ACT_KEYS), ws
 
 
+def _grad_wanted(*ts) -> bool:
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in ts)
+
+
+def _gains_bases(spec: LQGSpec, mats: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+    """``mats`` with the actor's seven matrices replaced by their (S|1, r, c) base matrices, taken from the spec through
+    differentiable views.  The library sees the same pointers and strides (a time-invariant array has a stride-0 time axis),
+    so the gains call is the same; the gradient of a base matrix flows back to the spec's array by autograd."""
+    out = dict(mats)
+    for k in ACT_KEYS:
+        M4 = _as4(getattr(spec, k))
+        if not is_time_invariant(M4):
+            raise NotImplementedError(
+                "lqg_b200: gradients of lqr.backward / kf.forward are implemented for time-invariant specs (stride-0 time "
+                "axis, as built by lqg_b200.utils.time_stack); materialised time-varying arrays only support the forward pass.")
+        out[k] = _row_major(M4[:, 0])
+    return out
+
+
+class _GainsFn(torch.autograd.Function):
+    """The gains of one sweep with the CUDA adjoint (lqgk_gains_vjp_*) as backward: ``kind`` "lqr" returns lqr_backward's
+    (L, l, H), "kf" kf_forward's K.  The forward is the gains call itself.
+
+    ``fixed``: what the call reads that is not differentiated; ``names``: the keys of the differentiable inputs ``mats`` --
+    (S|1, r, c) base matrices: A, B, Q, R and Qf for the Riccati sweep, A, F, V, W and Sigma0 for the Kalman sweep.  ``l`` and
+    ``H`` are not differentiable: ``l`` is zero in every reference model (no affine cost terms) and ``H`` is a by-product."""
+
+    @staticmethod
+    def forward(ctx, kind, dims, eps, fixed, names, *mats):
+        lib = abi.load_library()
+        act = {**fixed, **dict(zip(names, mats))}
+        sigma0 = act.pop("Sigma0", None)
+        dev = act["A"].device
+        ws = workspace(dev, lib.workspace_bytes(dims, abi.MODE_GAINS, 0))
+        ctx.kind, ctx.dims, ctx.eps, ctx.names = kind, dims, eps, names
+        ctx.act, ctx.sigma0 = act, sigma0
+        ctx.shapes = [m.shape for m in mats]
+        if kind == "kf":
+            return lib.kf_forward(dims, act, sigma0=sigma0, ws=ws, stream=_stream(dev))
+        L, l, H = lib.lqr_backward(dims, act, eps=eps, ws=ws, stream=_stream(dev))
+        ctx.mark_non_differentiable(l, H)
+        return L, l, H
+
+    @staticmethod
+    def backward(ctx, bar, *_l_H_bar):
+        if bar is None:
+            return (None,) * (5 + len(ctx.shapes))
+        lib = abi.load_library()
+        dev = bar.device
+        ws = workspace(dev, lib.workspace_bytes(ctx.dims, abi.MODE_GAINS_VJP, 0))
+        act = {k: ctx.act[k] for k in ACT_KEYS + ("Qf",) if k in ctx.act}   # (the adjoint reads no affine terms)
+        g, gs = lib.gains_vjp(ctx.dims, act, sigma0=ctx.sigma0, eps=ctx.eps, L_bar=bar if ctx.kind == "lqr" else None,
+                              K_bar=bar if ctx.kind == "kf" else None, want=[k for k in ctx.names if k != "Sigma0"], ws=ws,
+                              stream=_stream(dev))
+        g["Sigma0"] = gs
+        # the kernels sum over time; an input shared by the samples (leading 1) gets the sum over samples
+        out = [g[k].sum(0, keepdim=True) if (shp[0] == 1 and g[k].shape[0] != 1) else g[k] for k, shp in zip(ctx.names, ctx.shapes)]
+        return (None,) * 5 + tuple(out)
+
+
 def lqr_backward(spec: LQGSpec, eps: float = 1e-8):
-    """CUDA backward Riccati sweep.  Returns L, l, H shaped like the reference ((T,u,b) or (S,T,u,b))."""
+    """CUDA backward Riccati sweep.  Returns L, l, H shaped like the reference ((T,u,b) or (S,T,u,b)).
+
+    L is differentiable with respect to the spec's A, B, Q, R and Qf (time-invariant specs without a cross cost P); l and H
+    are not."""
     lib, dims, mats, ws = _gains_call(spec)
     # affine terms are always handed to the kernel (zeros in every reference model): no host-side "is it zero?" sync
     for k, tr in (("q", 1), ("r", 1), ("P", 2)):
@@ -175,17 +238,33 @@ def lqr_backward(spec: LQGSpec, eps: float = 1e-8):
         mats["qf"] = (spec.qf if spec.qf.dim() == 2 else spec.qf.unsqueeze(0)).contiguous()
     if spec.Qf is not None:
         mats["Qf"] = _untimed(spec.Qf, spec.A.dtype)
-    L, l, H = lib.lqr_backward(dims, mats, eps=eps, ws=ws, stream=_stream(spec.A.device))
+    if _grad_wanted(spec.A, spec.B, spec.Q, spec.R, spec.Qf):
+        _check_no_cross_cost(spec)
+        mats = _gains_bases(spec, mats)
+        names = ("A", "B", "Q", "R") + (("Qf",) if "Qf" in mats else ())
+        fixed = {k: v for k, v in mats.items() if k not in names}
+        L, l, H = _GainsFn.apply("lqr", dims, eps, fixed, names, *(mats[k] for k in names))
+    else:
+        L, l, H = lib.lqr_backward(dims, mats, eps=eps, ws=ws, stream=_stream(spec.A.device))
     if spec.A.dim() == 3:
         L, l, H = L[0], l[0], H[0]
     return L, l, H
 
 
 def kf_forward(spec: LQGSpec, Sigma0: Optional[torch.Tensor]):
-    """CUDA forward Kalman-gain sweep.  Returns K shaped (T,b,y) or (S,T,b,y)."""
+    """CUDA forward Kalman-gain sweep.  Returns K shaped (T,b,y) or (S,T,b,y).
+
+    K is differentiable with respect to the spec's A, F, V, W and Sigma0 (time-invariant specs)."""
     lib, dims, mats, ws = _gains_call(spec)
     s0 = None if Sigma0 is None else _untimed(Sigma0, spec.A.dtype)
-    K = lib.kf_forward(dims, mats, sigma0=s0, ws=ws, stream=_stream(spec.A.device))
+    if _grad_wanted(spec.A, spec.F, spec.V, spec.W, Sigma0):
+        mats = _gains_bases(spec, mats)
+        names = ("A", "F", "V", "W") + (("Sigma0",) if s0 is not None else ())
+        mats["Sigma0"] = s0
+        fixed = {k: v for k, v in mats.items() if k not in names}
+        K = _GainsFn.apply("kf", dims, 0.0, fixed, names, *(mats[k] for k in names))
+    else:
+        K = lib.kf_forward(dims, mats, sigma0=s0, ws=ws, stream=_stream(spec.A.device))
     return K[0] if spec.A.dim() == 3 else K
 
 
