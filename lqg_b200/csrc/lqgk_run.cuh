@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <numeric>
 #include <vector>
 
 #include "../../include/lqgk.h"
@@ -609,12 +610,22 @@ int run(const Call& c) {
   const size_t slice_bytes = up(p.bytes, ALIGN);
   const int Tn = d.T, N = d.N;
   const bool vjp = c.mode == LQGK_MODE_VJP;
-  // time segments of the launch sequence of a chunk of n samples (see below)
+  // Time segments of the launch sequence of a chunk of n samples (see below): segment g covers the checkpoint segments
+  // [kb[g], kb[g + 1]).  Its inner boundaries fall on multiples of `al` checkpoint segments, where the record chunks of
+  // k_trial_fwd (trial_tb steps) start, so that every launch of it sums the log-density over the same chunks as one launch
+  // over all segments: the pipelined sequence computes what the one-segment sequence computes.
+  const TrialGeom tg = trial_geom<DM>(N, Tn);
   auto segments = [&](int n) {
-    if (is_big<DM>() || !vjp || g_aux_streams == 0 || n > g_pipe_max_samples) return 1;
-    return std::max(1, std::min(g_pipe_segments, trial_geom<DM>(N, Tn).nseg));
+    const int G = is_big<DM>() || !vjp || g_aux_streams == 0 || n > g_pipe_max_samples ? 1 : std::max(1, std::min(g_pipe_segments, tg.nseg));
+    const int al = trial_tb<DM>() / std::gcd(tg.CK, trial_tb<DM>());
+    std::vector<int> kb{0};
+    for (int g = 1; g <= G; ++g) {
+      const int k = g == G ? tg.nseg : (int)((long long)g * tg.nseg / G) / al * al;
+      if (k > kb.back()) kb.push_back(k);
+    }
+    return kb;
   };
-  const bool pipelined = segments((int)((size_t)d.S - ((size_t)d.S - 1) / Sc * Sc)) > 1;   // (the last chunk is the smallest)
+  const bool pipelined = segments((int)((size_t)d.S - ((size_t)d.S - 1) / Sc * Sc)).size() > 2;   // (the last chunk is the smallest)
   const int nstreams = (ns > 1 ? ns : 0) + (pipelined ? 3 * ns : 0);
   if (nstreams > 0) {
     if (int rcp = g_pool.acquire(nstreams, c.stream)) return rcp;
@@ -723,8 +734,10 @@ int run(const Call& c) {
     //   t down: trial_rev (st) -> cov_seq_rev (x1) -> contraction (x2) -> kf_rev (x3);  lqr_rev (t up) follows on x2
     // Carries between segments: P_t, C_t and the checkpoints of c_t are stored per step anyway (adjoint linearisation points);
     // the adjoint carries (cb, Cb, Pnb) go through three small buffers.  G = 1 (forward only, large systems, kernel overlap
-    // off, chunks above g_pipe_max_samples, T within one checkpoint interval) is the same sequence on the chunk's stream.
-    const int G = segments(n);
+    // off, chunks above g_pipe_max_samples, T within one checkpoint interval or one multiple `al` of it) is the same sequence
+    // on the chunk's stream.
+    const std::vector<int> kb = segments(n);
+    const int G = (int)kb.size() - 1;
     cudaStream_t x1 = st, x2 = st, x3 = st;
     if (G > 1) {
       const int a = aux0 + 3 * (chunk_idx % ns);
@@ -732,9 +745,8 @@ int run(const Call& c) {
       x2 = g_pool.streams[a + 1];
       x3 = g_pool.streams[a + 2];
     }
-    const TrialGeom tg = trial_geom<DM>(N, Tn);
-    std::vector<int> kb(G + 1), tb(G + 1);   // segment g: checkpoint segments [kb[g], kb[g + 1]), steps [tb[g], tb[g + 1])
-    for (int g = 0; g <= G; ++g) { kb[g] = (int)((long long)g * tg.nseg / G); tb[g] = std::min(Tn, kb[g] * tg.CK); }
+    std::vector<int> tb(G + 1);   // segment g: steps [tb[g], tb[g + 1])
+    for (int g = 0; g <= G; ++g) tb[g] = std::min(Tn, kb[g] * tg.CK);
     dep(st, x1);                                 // pack done -> kf_fwd on x1 beside lqr_fwd on st
     if ((rc = k.template lqr_fwd<false>(st))) return rc;
     dep(st, x2);                                 // L complete -> covariance pass

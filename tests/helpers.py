@@ -58,29 +58,43 @@ def jittered_params(name, S, seed, scale=0.25):
 
 
 class Case:
-    """S jittered parameter samples of one model, N simulated trials (from sample 0), oracle results in float64."""
+    """S jittered parameter samples of one model, N simulated trials, oracle results in float64.
 
-    def __init__(self, name, S, T, N, d=None, seed=0, weights=False, want_grad=True):
+    The trials are simulated from sample 0 and shared by all samples, or with `per_sample_data` one data set per sample,
+    simulated from that sample's own parameters (X[S, N, T+1, d]; the library then sees x_sample_stride != 0).  The
+    cotangents of the per-trial log-likelihoods are 1 (default), uniform(0.5, 1.5) (`weights`) or given explicitly (`w`,
+    [S, N]); the oracle's gradient is that of sum_i w[s, i] ll[s, i] for every sample s."""
+
+    def __init__(self, name, S, T, N, d=None, seed=0, weights=False, want_grad=True, per_sample_data=False, w=None):
         self.name, self.S, self.T, self.N = name, S, T, N
         x, b, u, y = MODEL_DIMS[name]
         self.d = d if d is not None else x
         self.dims = (x, b, u, y, self.d)
+        self.per_sample_data = per_sample_data
         self.params = jittered_params(name, S, seed)
         self.mats = [model_mats(name, **kw) for kw in self.params]
-        sa, sd = O.make_system(self.mats[0], T)
         rng = np.random.default_rng(seed + 1)
-        X = O.simulate(sa, sd, N, rng)[..., :self.d]
+        if per_sample_data:
+            X = np.stack([O.simulate(*O.make_system(m, T), N, rng) for m in self.mats])[..., :self.d]
+        else:
+            sa, sd = O.make_system(self.mats[0], T)
+            X = O.simulate(sa, sd, N, rng)[..., :self.d]
         self.X = X.astype(np.float32)                       # what the library sees
         X64 = self.X.astype(np.float64)
-        self.w = rng.uniform(0.5, 1.5, (S, N)) if weights else None
+        if w is not None:
+            self.w = np.asarray(w, dtype=np.float64)
+            assert self.w.shape == (S, N), self.w.shape
+        else:
+            self.w = rng.uniform(0.5, 1.5, (S, N)) if weights else None
         self.ll = np.zeros((S, N))
         self.ga, self.gd = [], []
         for s, m in enumerate(self.mats):
+            Xs = X64[s] if per_sample_data else X64
             if want_grad:
-                ll, (ga, gd) = AD.value_and_grad(m[0], m[1], X64, w=None if self.w is None else self.w[s])
+                ll, (ga, gd) = AD.value_and_grad(m[0], m[1], Xs, w=None if self.w is None else self.w[s])
                 self.ga.append(ga); self.gd.append(gd)
             else:
-                ll, _ = AD.forward(m[0], m[1], X64)
+                ll, _ = AD.forward(m[0], m[1], Xs)
             self.ll[s] = ll
 
     def tensors(self, device, dtype):
@@ -90,8 +104,18 @@ class Case:
                for k in abi.DYN_KEYS}
         return act, dyn
 
-    def lqgk_dims(self):
-        return abi.LqgkDims(self.S, self.N, self.T, *self.dims)
+    def x_tm(self, lib, device):
+        """The observations in the library's time-major layout: [T+1, N, d], or [S, T+1, N, d] with one set per sample."""
+        st = stream_of(device)
+        if not self.per_sample_data:
+            return lib.pack_obs(torch.tensor(self.X, device=device), stream=st)
+        return torch.stack([lib.pack_obs(torch.tensor(X, device=device), stream=st) for X in self.X])
+
+    def lqgk_dims(self, S=None):
+        """The call's dims (S systems, default the case's samples); with per-sample data, the stride between the data sets
+        of x_tm(), which the workspace size depends on."""
+        stride = (self.T + 1) * self.N * self.d if self.per_sample_data else 0
+        return abi.LqgkDims(self.S if S is None else S, self.N, self.T, *self.dims, stride)
 
 
 def workspace(lib, dims, mode, device, max_chunk=0):
@@ -114,7 +138,7 @@ def check_vjp(lib, device, case: Case, dtype=torch.float32, max_chunk=0, ll_rtol
     Gradient criterion: max-abs error <= g_rtol * max-abs of that matrix' oracle gradient (per sample)."""
     dims = case.lqgk_dims()
     act, dyn = case.tensors(device, dtype)
-    x_tm = lib.pack_obs(torch.tensor(case.X, device=device), stream=stream_of(device))
+    x_tm = case.x_tm(lib, device)
     ws = workspace(lib, dims, abi.MODE_VJP, device, max_chunk)
     ll_bar = None if case.w is None else torch.tensor(case.w, dtype=dtype, device=device)
     ll, oa, od, _ = lib.loglik_vjp(dims, act, dyn, x_tm, ll_bar=ll_bar, ws=ws, stream=stream_of(device))
@@ -136,29 +160,38 @@ def check_vjp(lib, device, case: Case, dtype=torch.float32, max_chunk=0, ll_rtol
     return worst
 
 
-def check_vjp_tiled(lib, device, case: Case, reps: int, dtype=torch.float32, ll_rtol=1e-4, g_rtol=1e-3):
-    """check_vjp with the case's samples repeated `reps` times (S * reps systems in one call): reaches sample counts whose
-    kernels differ from the small-batch ones (thread-per-sample covariance kernels above 1,024 samples) at the oracle cost of S."""
+def check_vjp_tiled(lib, device, case: Case, reps: int = 1, dtype=torch.float32, ll_rtol=1e-4, g_rtol=1e-3, total=None, max_chunk=0):
+    """check_vjp on `total` systems in one call (default S * reps), system k being sample k mod S of the case, with that
+    sample's data set when the case has one per sample: reaches sample counts whose kernels differ from the small-batch ones
+    (thread-per-sample covariance kernels above 1,024 samples; several chunks with `max_chunk`) at the oracle cost of S.
+    Every system is compared with the oracle."""
     S = case.S
-    dims = abi.LqgkDims(S * reps, case.N, case.T, *case.dims)
+    total = S * reps if total is None else total
+    idx = torch.arange(total, device=device) % S
+    dims = case.lqgk_dims(total)
     act, dyn = case.tensors(device, dtype)
-    act = {k: v.repeat(reps, 1, 1).contiguous() for k, v in act.items()}
-    dyn = {k: v.repeat(reps, 1, 1).contiguous() for k, v in dyn.items()}
-    x_tm = lib.pack_obs(torch.tensor(case.X, device=device), stream=stream_of(device))
-    ws = workspace(lib, dims, abi.MODE_VJP, device)
-    ll_bar = None if case.w is None else torch.tensor(case.w, dtype=dtype, device=device).repeat(reps, 1).contiguous()
+    act = {k: v[idx].contiguous() for k, v in act.items()}
+    dyn = {k: v[idx].contiguous() for k, v in dyn.items()}
+    x_tm = case.x_tm(lib, device)
+    if case.per_sample_data:
+        x_tm = x_tm[idx].contiguous()
+    ws = workspace(lib, dims, abi.MODE_VJP, device, max_chunk)
+    ll_bar = None if case.w is None else torch.tensor(case.w, dtype=dtype, device=device)[idx].contiguous()
     ll, oa, od, _ = lib.loglik_vjp(dims, act, dyn, x_tm, ll_bar=ll_bar, ws=ws, stream=stream_of(device))
     if device.type == "cuda":
         torch.cuda.synchronize(device)
     ll = ll.double().cpu().numpy()
-    for r in (0, reps // 2, reps - 1):
-        assert np.allclose(ll[r * S:(r + 1) * S], case.ll, rtol=ll_rtol)
-        for s in range(S):
-            floor = 1e-9 * max(max(np.abs(case.ga[s][k]).max() for k in abi.ACTOR_KEYS), max(np.abs(case.gd[s][k]).max() for k in abi.DYN_KEYS))
-            for keys, out, ref in ((abi.ACTOR_KEYS, oa, case.ga), (abi.DYN_KEYS, od, case.gd)):
-                for k in keys:
-                    err = np.abs(out[k][r * S + s].double().cpu().numpy() - ref[s][k]).max()
-                    assert err <= g_rtol * np.abs(ref[s][k]).max() + floor, (k, r, s, err)
+    oa = {k: v.double().cpu().numpy() for k, v in oa.items()}
+    od = {k: v.double().cpu().numpy() for k, v in od.items()}
+    floor = [1e-9 * max(max(np.abs(case.ga[s][k]).max() for k in abi.ACTOR_KEYS), max(np.abs(case.gd[s][k]).max() for k in abi.DYN_KEYS))
+             for s in range(S)]
+    for j in range(total):
+        s = j % S
+        assert np.allclose(ll[j], case.ll[s], rtol=ll_rtol), (j, rel_err(ll[j], case.ll[s]))
+        for keys, out, ref in ((abi.ACTOR_KEYS, oa, case.ga), (abi.DYN_KEYS, od, case.gd)):
+            for k in keys:
+                err = np.abs(out[k][j] - ref[s][k]).max()
+                assert err <= g_rtol * np.abs(ref[s][k]).max() + floor[s], (k, j, s, err)
 
 
 def check_param_vjp(lib, device, case: Case, dtype=torch.float32, ll_rtol=1e-4, g_rtol=1e-3):
@@ -167,7 +200,7 @@ def check_param_vjp(lib, device, case: Case, dtype=torch.float32, ll_rtol=1e-4, 
     differences of the oracle's constructor).  Criterion per sample: |g - g_ref| <= g_rtol * |g_ref| + 1e-4 * max|g_ref|."""
     dims = case.lqgk_dims()
     act, dyn = case.tensors(device, dtype)
-    x_tm = lib.pack_obs(torch.tensor(case.X, device=device), stream=stream_of(device))
+    x_tm = case.x_tm(lib, device)
     ws = workspace(lib, dims, abi.MODE_VJP, device)
     ll, oa, od, _ = lib.loglik_vjp(dims, act, dyn, x_tm, ws=ws, stream=stream_of(device))
     if device.type == "cuda":
@@ -194,7 +227,7 @@ def check_param_vjp(lib, device, case: Case, dtype=torch.float32, ll_rtol=1e-4, 
 def check_fwd(lib, device, case: Case, dtype=torch.float32, max_chunk=0, ll_rtol=1e-4):
     dims = case.lqgk_dims()
     act, dyn = case.tensors(device, dtype)
-    x_tm = lib.pack_obs(torch.tensor(case.X, device=device), stream=stream_of(device))
+    x_tm = case.x_tm(lib, device)
     ws = workspace(lib, dims, abi.MODE_FWD, device, max_chunk)
     ll = lib.loglik_fwd(dims, act, dyn, x_tm, ws=ws, stream=stream_of(device))
     if device.type == "cuda":
